@@ -12,9 +12,9 @@ ends a step, inside the step's CUDA graph: this library's peer-memory kernel, `-
 value  : scenes/s, inputs resident in HBM.  Every step is one CUDA-graph replay; `--pipeline` (default 24) steps are in
          flight on separate streams with their own graphs and buffers (a step chains latency-bound sampling stages that
          keep a few SMs busy for milliseconds and short throughput-bound stages, so steps overlap).  Timing: after
-         max(W, 2*pipeline) warm-up steps, `--brackets` (5) brackets of K*reps steps each (reps chosen so a bracket lasts
-         >= 0.5 s), one CUDA-event pair per bracket, barrier + synchronize on both sides, L2 flushed before every step,
-         max over ranks per bracket, MEDIAN bracket reported; ms_per_step = that bracket / its steps.
+         max(W, 2*pipeline) warm-up steps, `--brackets` (5) brackets of exactly K steps each, one CUDA-event pair per
+         bracket, barrier + synchronize on both sides, L2 flushed before every step, max over ranks per bracket, MEDIAN
+         bracket reported; ms_per_step = that bracket / K.
 e2e    : the same brackets through the public API with HOST buffers: pinned H2D copy of the batch into the graph's
          input + the step + D2H read of the gathered detection blocks inside the timed region.
 config.latency_ms_single_step: one step at a time (sync after each), the library's latency mode (SABackbone
@@ -22,6 +22,9 @@ config.latency_ms_single_step: one step at a time (sync after each), the library
 roofline: time-weighted tensor-pipe figure over ALL grouped-MLP kernels of one step (the kernels that dominate the
          step's SM-time), each timed live with CUDA events; roofline_fps: the layer-1 D-FPS chain (ns per round).
 cpu_baseline: the CPU restatement (oracle/, fp32 BLAS MLP) on a bounded sample of the same workload.
+--dump-outputs DIR: after the timed brackets, what the last timed step returned to its caller is written as DIR/<name>.npy
+         (float32; integer outputs as float64): the per-layer points, features and sample indices of rank 0 and the
+         detections of all ranks.  Inputs and weights are seeded, so two builds can be compared output for output.
 clocks : sampled in-process through NVML from before the first bracket to after the last one (no nvidia-smi start-up
          inside a bracket); median / reasons are over the samples that fall inside timed brackets.
 
@@ -34,7 +37,6 @@ if that library is absent it falls back to the CPU port.  Its cpu_baseline objec
 import argparse
 import importlib
 import json
-import math
 import os
 import subprocess
 import sys
@@ -310,7 +312,6 @@ def main():
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--brackets", type=int, default=5, help="timed brackets per leg; the median is reported")
-    ap.add_argument("--min-bracket-s", type=float, default=0.5, help="a bracket runs K*reps steps with reps chosen to last this long")
     ap.add_argument("--ffps-mode", default="direct", choices=["direct", "matrix", "fused"])
     ap.add_argument("--mlp-mode", default="tc", choices=["tc", "fp32"])
     ap.add_argument("--gather-in-kernel", type=int, default=1, help="1: first conv of unfused SA scales gathers its operand itself")
@@ -327,6 +328,8 @@ def main():
                     help="N > 1: the per-step all-gather as this library's peer-memory kernel (default) or as ncclAllGather")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-scenes", type=int, default=2)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned as DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
 
@@ -482,9 +485,11 @@ def main():
     host_in = torch.from_numpy(pts_np).pin_memory()
     host_out = [torch.empty((gathers[k].raw.numel(),), dtype=torch.uint8).pin_memory() for k in range(P)]
 
+    last = {}
+
     def one_step(i, e2e):
         k = i % P
-        runners[k](host_in if e2e else None)      # e2e: pinned H2D into the graph's static input first
+        last["k"], last["out"] = k, runners[k](host_in if e2e else None)      # e2e: pinned H2D into the graph's static input first
         if e2e:
             host_out[k].copy_(gathers[k].raw, non_blocking=True)   # all ranks' detection blocks + counts
 
@@ -517,9 +522,7 @@ def main():
 
     warm = max(args.warmup, 2 * P)
     bracket(warm, False, timed=False)
-    est = bracket(args.steps, False, timed=False) / args.steps                 # ms per step, same on all ranks (max-reduced)
-    reps = max(1, int(math.ceil(args.min_bracket_s * 1e3 / (est * args.steps))))
-    nsteps = args.steps * reps
+    nsteps = args.steps
     val_ms = sorted(bracket(nsteps, False) for _ in range(max(1, args.brackets)))
     total_ms = val_ms[len(val_ms) // 2]
 
@@ -528,6 +531,8 @@ def main():
     e2e_all = sorted(bracket(nsteps, True) for _ in range(max(1, args.brackets)))
     e2e_ms = e2e_all[len(e2e_all) // 2]
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last["out"][0], gathers[last["k"]].result())
 
     # ---- single-step latency: one step at a time, sync after each, latency-mode network --------------------
     lat_runner = None
@@ -610,10 +615,10 @@ def main():
                                        "graph (SABackbone latency_mode=True) / the throughput graph used for `value`",
                        "brackets": len(val_ms), "steps_per_bracket": nsteps, "warmup_effective": warm,
                        "bracket_ms": val_ms, "e2e_bracket_ms": e2e_all,
-                       "timing": "median of %d brackets of %d steps (= steps x %d, >= %.1f s each); one CUDA-event pair per bracket "
+                       "timing": "median of %d brackets of %d steps; one CUDA-event pair per bracket "
                                  "(L2 flushes included), barrier + synchronize on both sides, max over ranks per bracket; every step is "
                                  "one CUDA-graph replay incl. the ncclAllGather, %d step pipelines on separate streams"
-                                 % (len(val_ms), nsteps, reps, args.min_bracket_s, P)},
+                                 % (len(val_ms), nsteps, P)},
             "e2e": {"value": scenes / (e2e_ms * 1e-3), "unit": UNIT,
                     "h2d_bytes_per_step": int(host_in.numel() * 4), "d2h_bytes_per_step": int(host_out[0].numel())},
             "gpu_launches": launches_per_step * args.steps,
@@ -659,6 +664,26 @@ def main():
         sys.stdout.flush()
         sys.stderr.flush()
         os._exit(0)
+
+
+def dump_outputs(out_dir, forward_out, detections, limit_bytes=64 * 10 ** 6):
+    """Writes a step's outputs as <out_dir>/<name>.npy: xyz_<l>, features_<l>, fps_idx_<l> per layer of the backbone
+    (None entries skipped), detection_boxes [B,100,9] and detection_counts [B].  Floating outputs are float32, integer
+    ones float64 (exact)."""
+    arrays = {}
+    for prefix, tensors in zip(("xyz", "features", "fps_idx"), forward_out):
+        for i, t in enumerate(tensors):
+            if t is not None:
+                arrays["%s_%d" % (prefix, i)] = t
+    arrays["detection_boxes"], arrays["detection_counts"] = detections
+    arrays = {k: t.detach().cpu().numpy() for k, t in arrays.items()}
+    arrays = {k: a.astype(np.float32 if a.dtype.kind == "f" else np.float64) for k, a in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > limit_bytes:
+        raise SystemExit("bench.py: the step's outputs take %d bytes, more than the %d a dump may hold" % (total, limit_bytes))
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
 
 
 def run_reference(args, torch, pkg, arch, params, head_params, pts_np, rank, world, dev, sampler):

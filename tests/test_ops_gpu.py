@@ -1,5 +1,6 @@
 """GPU parity tests (-m gpu): every operator of libssd3d.so, called through the tf_ops surface (ctypes ->
-C ABI), against (a) the CPU oracle and (b) the reference's own kernels run live (oracle/_ref).
+C ABI), against (a) the CPU oracle and (b) the outputs of the reference's own kernels on the same inputs (ref_ops:
+stored under tests/golden/ref_kernels/, see oracle/ref_golden.py).
 Integer outputs must be bit-exact; fp32 copies / interpolation bit-exact; the MLP within 1e-3 relative."""
 import importlib
 

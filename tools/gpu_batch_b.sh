@@ -18,6 +18,6 @@ for a in "dyn=1 slots=4 wg=1" "dyn=1 slots=3 wg=1" "dyn=1 slots=2 wg=2" "dyn=1 s
 timeout 900 compute-sanitizer --tool memcheck --error-exitcode 9 python tools/sanitize_probe.py > $O/r02_sanitizer_memcheck.txt 2>&1; echo "exit $?" >> $O/r02_sanitizer_memcheck.txt
 timeout 900 compute-sanitizer --tool racecheck --error-exitcode 9 python tools/sanitize_probe.py > $O/r02_sanitizer_racecheck.txt 2>&1; echo "exit $?" >> $O/r02_sanitizer_racecheck.txt
 # launch list of one eager step (throughput schedule and latency schedule)
-timeout 600 ncu --metrics gpu__time_duration.sum --clock-control none --csv --log-file $O/launches_r02.csv python bench.py --no-graph --pipeline 1 --no-cpu-baseline --steps 3 --warmup 3 --brackets 1 --min-bracket-s 0 > $O/ncu_bench.log 2>&1
+timeout 600 ncu --metrics gpu__time_duration.sum --clock-control none --csv --log-file $O/launches_r02.csv python bench.py --no-graph --pipeline 1 --no-cpu-baseline --steps 3 --warmup 3 --brackets 1 > $O/ncu_bench.log 2>&1
 cat $O/fused_ab.log; tail -3 $O/sweep_fps.log $O/sweep_bq.log $O/tc_prof.log $O/fused_prof.log
 tail -4 $O/r02_sanitizer_memcheck.txt $O/r02_sanitizer_racecheck.txt

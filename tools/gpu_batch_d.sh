@@ -7,7 +7,7 @@ mkdir -p $O
 timeout 900 python -m pytest tests -m gpu -q 2>&1 | tail -15 > $O/tests_final.log
 python bench.py --impl reference --steps 10 > $O/bench_ref_final.json 2> $O/bench_ref_final.err
 python bench.py > $O/bench_final.json 2> $O/bench_final.err
-BENCH1="python bench.py --no-graph --pipeline 1 --no-cpu-baseline --steps 3 --warmup 3 --brackets 1 --min-bracket-s 0"
+BENCH1="python bench.py --no-graph --pipeline 1 --no-cpu-baseline --steps 3 --warmup 3 --brackets 1"
 timeout 600 ncu --metrics gpu__time_duration.sum --clock-control none --csv --log-file $O/launches_final.csv $BENCH1 > $O/ncu_bench_final.log 2>&1
 NCU="ncu --set full --clock-control none --import-source on --launch-count 1"
 cap() {  # name, kernel regex, launch-skip
