@@ -7,6 +7,8 @@ torch CUDA tensors instead of TF tensors.  What TF resolved through variable sco
 convs with batch-statistics BatchNorm and updates the moving statistics in place (tf_util.py:424-444); the fused
 inference kernels fold BN and therefore serve is_training=False only.
 """
+from typing import NamedTuple
+
 import torch
 
 from . import config as _cfg
@@ -14,8 +16,7 @@ from . import tf_ops
 from .params import prepare
 
 
-def _conv(pp, scope, x, bn=True, relu=True, pool=1, rowmask=None):
-    f = pp.conv(scope, bn)
+def _conv(f, x, relu=True, pool=1, rowmask=None):
     return tf_ops.linear_bn_relu(x, f.w, f.scale, f.shift, relu=relu, pool=pool, rowmask=rowmask, cin=f.cin)
 
 
@@ -33,22 +34,27 @@ def _conv_train(pp, scope, x, bn, bn_decay, relu=True):
                            decay=0.9 if bn_decay is None else float(bn_decay), relu=relu)[0]
 
 
+def _ball_query(xyz, new_xyz, radius_list, nsample_list, dilated_group, want_units=False):
+    """The neighbour lists of every shell (:137-145) -> (idx_list, cnt_list, units_list); units_list holds the unit lists
+    of the grouped MLPs when want_units (None where query_ball_point_multi has none), else Nones."""
+    nscale = len(radius_list)
+    min_r = [0.0 if (i == 0 or not dilated_group) else radius_list[i - 1] for i in range(nscale)]   # :137-141
+    if nscale <= 4:                                                       # one pass over the candidates for all shells
+        res = tf_ops.query_ball_point_multi(min_r, radius_list, nsample_list, xyz, new_xyz, dilated_group,
+                                            return_units=want_units)
+        return res[0], res[1], res[2] if want_units else [None] * nscale
+    res = [tf_ops.query_ball_point_dilated(min_r[i], radius_list[i], nsample_list[i], xyz, new_xyz) if dilated_group
+           else tf_ops.query_ball_point(radius_list[i], nsample_list[i], xyz, new_xyz) for i in range(nscale)]
+    return [r[0] for r in res], [r[1] for r in res], [None] * nscale
+
+
 def _group_and_mlp_train(pp, scope, xyz, points, new_xyz, radius_list, nsample_list, mlp_list, bn, bn_decay, dilated_group,
-                         use_agg, debug):
+                         use_agg):
     """Training-mode twin of _group_and_mlp: the literal op sequence of layers_util.py:137-185 (grouped tensor
     materialised once, conv -> batch-norm -> relu per layer, reduce_max, mask, concat, aggregation)."""
-    nscale = len(radius_list)
-    min_r = [0.0 if (i == 0 or not dilated_group) else radius_list[i - 1] for i in range(nscale)]
-    idx_list, cnt_list = tf_ops.query_ball_point_multi(min_r, radius_list, nsample_list, xyz, new_xyz, dilated_group) \
-        if nscale <= 4 else ([], [])
-    if nscale > 4:
-        for i in range(nscale):
-            a, c = (tf_ops.query_ball_point_dilated(min_r[i], radius_list[i], nsample_list[i], xyz, new_xyz) if dilated_group
-                    else tf_ops.query_ball_point(radius_list[i], nsample_list[i], xyz, new_xyz))
-            idx_list.append(a); cnt_list.append(c)
-    debug["idx"].append(idx_list); debug["cnt"].append(cnt_list)
+    idx_list, cnt_list, _ = _ball_query(xyz, new_xyz, radius_list, nsample_list, dilated_group)
     outs = []
-    for i in range(nscale):
+    for i in range(len(radius_list)):
         g = tf_ops.group_concat(xyz, points, new_xyz, idx_list[i])                                  # :160-165
         for j in range(len(mlp_list[i])):
             g = _conv_train(pp, "%s/conv%d_%d" % (scope, i, j), g, bn, bn_decay)                    # :167-176
@@ -56,7 +62,7 @@ def _group_and_mlp_train(pp, scope, xyz, points, new_xyz, radius_list, nsample_l
     new_points = outs[0] if len(outs) == 1 else torch.cat(outs, dim=-1)
     if use_agg:
         new_points = _conv_train(pp, scope + "/ensemble", new_points, bn, bn_decay)                 # :183-185
-    return new_points
+    return new_points, idx_list, cnt_list
 
 
 _CONSTS = {}
@@ -124,212 +130,160 @@ COMPACT_GROUPS = True      # fused SA scales convolve only the 8-row units that 
 HOIST_EXPAND_MIN_K = 256   # hoisted second convs at least this wide materialise their operand (tf_ops.hoist_expand_split)
 
 
-class _Hoisted:
-    """The per-point table of the hoisted first convs of a layer (see pointnet_sa_module_msg)."""
-    __slots__ = ("scales", "z", "zoffs", "wxs", "stacks")
+class _Scale(NamedTuple):
+    """Route of one scale's grouped MLP."""
+    stack: object     # FusedStack: the whole scale in one kernel (of the convs after the hoisted one); None: conv by conv
+    hoisted: bool     # the first conv comes from the layer's per-point table z
+    first: str        # tensor cores, conv by conv: how the first conv not in z gets its operand -- "gather" (in the kernel's
+                      # operand load, linear_tc_gather), "split" (group_concat_split), "hoisted" (in the kernel, from z:
+                      # linear_tc_hoisted), "expand" (from z, materialised: hoist_expand_split); otherwise None
+    units: bool       # convolve only the 8-row units that hold distinct neighbours, pool them into the concat buffer
+    convs: tuple      # FoldedConvs of the convs not in z
 
 
-def _prepare_hoist(pp, scope, mlp_list, bn, c_feat, stacks, gather_in_kernel, hoist_first):
-    nscale = len(mlp_list)
-    h = _Hoisted()
-    # hoist_first: 0 off, 1 layer-by-layer scales only, 2 all.  An xyz-only cloud (c_feat == 0) has no feature part to
+class _Plan(NamedTuple):
+    """Route of the grouped MLPs of one pointnet_sa_module_msg call (see _plan)."""
+    tc: bool          # tensor-core route (else fp32)
+    scales: list      # a _Scale per scale
+    zconv: object     # FoldedConv of the per-point table z = the feature part of every hoisted first conv (None: none)
+    hoist: dict       # hoisted scale -> (its first column in z, wx = its Wx * s1 (3, n1))
+    agg: object       # FoldedConv of the aggregation conv, or None
+    split: bool       # the scales also write the aggregation conv's split bf16 operand (else split_rows of the concat)
+
+    def __str__(self):
+        return repr(self._replace(hoist={i: (zoff, "wx%s" % list(wx.shape)) for i, (zoff, wx) in self.hoist.items()}))
+
+
+def _plan(pp, scope, mlp_list, nsample_list, bn, c_feat, use_agg, mlp_mode, fuse_scale, gather_in_kernel, hoist_first):
+    scopes = [["%s/conv%d_%d" % (scope, i, j) for j in range(len(m))] for i, m in enumerate(mlp_list)]
+    agg = pp.conv(scope + "/ensemble", bn) if use_agg else None
+    # tensor cores: pooling widths the epilogue covers and 16-byte aligned column slices of the concat buffers
+    if not (mlp_mode == "tc" and all(k in (8, 16, 32, 64, 128) for k in nsample_list) and all(m[-1] % 8 == 0 for m in mlp_list)):
+        return _Plan(False, [_Scale(None, False, None, False, tuple(pp.conv(s, bn) for s in sc)) for sc in scopes],
+                     None, {}, agg, False)
+    stacks = [pp.fused_stack(sc, bn, c_feat + 3) if fuse_scale else None for sc in scopes]
+    # hoisted first convs: the feature part of conv0 of a scale, once per POINT (independent of the sampling).
+    # hoist_first: 0 off, 1 conv-by-conv scales only, 2 all.  An xyz-only cloud (c_feat == 0) has no feature part to
     # hoist: the first conv then runs in the grouped domain (linear_tc_gather / sa_mlp_fused accept c = 0).
-    h.scales = [i for i in range(nscale) if len(mlp_list[i]) >= 2 and (int(hoist_first) >= 2 or stacks[i] is None)] \
+    hoisted = [i for i, sc in enumerate(scopes) if len(sc) >= 2 and (int(hoist_first) >= 2 or stacks[i] is None)] \
         if (gather_in_kernel and hoist_first and c_feat > 0) else []
-    h.z = h.zoffs = h.wxs = None
-    h.stacks = {}
-    return h
+    zconv, hoist = None, {}
+    if hoisted:
+        zconv, wxs, n1s = pp.hoisted([scopes[i][0] for i in hoisted], bn, c_feat)
+        hoist = {i: (sum(n1s[:t]), wxs[t]) for t, i in enumerate(hoisted)}
+    scales = []
+    for i, sc in enumerate(scopes):
+        # unit lists come from the one-pass ball query; the fused kernels and the hoisted convs have *_units forms
+        units = COMPACT_GROUPS and len(scopes) <= 4 and (stacks[i] is not None or i in hoist)
+        convs = tuple(pp.conv(s, bn) for s in (sc[1:] if i in hoist else sc))
+        if stacks[i] is not None:
+            hstack = pp.fused_stack(sc[1:], bn, hoist[i][1].shape[1]) if i in hoist else None
+            scales.append(_Scale(stacks[i] if hstack is None else hstack, hstack is not None, None, units, convs))
+        elif i in hoist:
+            # wide layer: materialise the operand once (elementwise, memory speed), then the plain TMA-fed GEMM
+            expand = convs[0].kp >= HOIST_EXPAND_MIN_K and hoist[i][0] % 4 == 0 and zconv.cout % 4 == 0
+            scales.append(_Scale(None, True, "expand" if expand else "hoisted", units, convs))
+        else:
+            scales.append(_Scale(None, False, "gather" if gather_in_kernel else "split", units, convs))
+    return _Plan(True, scales, zconv, hoist, agg, agg is not None and not any(s.units for s in scales))
 
 
-def _compute_hoist(h, pp, scope, mlp_list, bn, points, stacks):
-    if not h.scales:
-        return
-    c_feat = points.shape[-1]
-    zconv, h.wxs, n1s = pp.hoisted(["%s/conv%d_0" % (scope, i) for i in h.scales], bn, c_feat)
+def _hoist_table(plan, points):
+    """The per-point table z of the hoisted first convs (b, n, sum n1)."""
     p_hi, p_lo = tf_ops.split_rows(points)
-    h.z, _ = tf_ops.linear_tc(p_hi, p_lo, zconv, relu=False, want_f32=True, want_split=False)
-    h.zoffs = [sum(n1s[:t]) for t in range(len(h.scales))]
-    for t, i in enumerate(h.scales):
-        if stacks[i] is not None:    # remaining convs of a fused scale
-            h.stacks[i] = pp.fused_stack(["%s/conv%d_%d" % (scope, i, j) for j in range(1, len(mlp_list[i]))], bn, n1s[t])
+    return tf_ops.linear_tc(p_hi, p_lo, plan.zconv, relu=False, want_f32=True, want_split=False)[0]
 
 
-def _group_and_mlp(pp, scope, xyz, points, new_xyz, radius_list, nsample_list, mlp_list, bn, dilated_group, use_agg,
-                   mlp_mode, stacks, hoist, gather_in_kernel, debug):
-    """Everything of pointnet_sa_module_msg after the sampling, for one block of query points new_xyz (b, m_q, 3):
-    ball queries (:137-145), grouping + MLP + max-pool + mask per scale (:157-180), concat + aggregation (:182-185)."""
-    bs = xyz.shape[0]
-    nscale = len(radius_list)
-    min_r = [0.0 if (i == 0 or not dilated_group) else radius_list[i - 1] for i in range(nscale)]   # :137-141
-    units_list = [None] * nscale
-    tc_path = (mlp_mode == "tc" and all(k in (8, 16, 32, 64, 128) for k in nsample_list) and all(m[-1] % 8 == 0 for m in mlp_list))
-    if nscale <= 4:   # one pass over the candidates for all shells
-        want_units = COMPACT_GROUPS and tc_path and (any(st is not None for st in stacks) or bool(hoist.scales))
-        res = tf_ops.query_ball_point_multi(min_r, radius_list, nsample_list, xyz, new_xyz, dilated_group, return_units=want_units)
-        idx_list, cnt_list = res[0], res[1]
-        if want_units:
-            units_list = res[2]
+def _fused_scale(s, xyz, points, z, zx, new_xyz, idx, cnt, out_f32, out_split, units):
+    """A whole scale in one kernel: gather (or the hoisted operand) + conv stack + max-pool + mask."""
+    if s.hoisted:
+        tf_ops.sa_mlp_fused_hoisted(xyz, z, *zx, new_xyz, idx, cnt, s.stack, out_f32=out_f32, out_split=out_split, units=units)
     else:
-        idx_list, cnt_list = [], []
-        for i in range(nscale):
-            if dilated_group:
-                a, c = tf_ops.query_ball_point_dilated(min_r[i], radius_list[i], nsample_list[i], xyz, new_xyz)
-            else:
-                a, c = tf_ops.query_ball_point(radius_list[i], nsample_list[i], xyz, new_xyz)
-            idx_list.append(a); cnt_list.append(c)
-    debug["idx"].append(idx_list); debug["cnt"].append(cnt_list)
-    # tensor-core path needs pooling widths the epilogue covers and 16-byte aligned column slices of the concat buffers
-    tc = tc_path
-    if tc:
-        # tensor-core path: every scale pools straight into its slice of the concat buffer (fp32 for the
-        # caller, split bf16 for the aggregation conv), activations stay split between layers
-        m_q = new_xyz.shape[1]
-        ctot = sum(m[-1] for m in mlp_list)
-        concat = torch.empty((bs, m_q, ctot), dtype=torch.float32, device=xyz.device)
-        # unit-list mode: the fused scales combine their 8-row units with atomicMax on the ZERO-FILLED fp32 concat buffer; the
-        # split copy the aggregation conv reads is then made once, from the finished buffer
-        # (layer-by-layer scales with a hoisted first conv take the same route through the *_units forms of their kernels)
-        use_units = [units_list[i] is not None and (stacks[i] is not None or i in hoist.scales) for i in range(nscale)]
-        compact = any(use_units)
-        if compact:
-            tf_ops.fill_zero(concat)
-        cat_hi = cat_lo = None
-        split_in_epilogue = use_agg and not compact
-        if split_in_epilogue:
-            ldc = tf_ops.round16(ctot)
-            mk = torch.zeros if ldc != ctot else torch.empty
-            cat_hi = mk((bs, m_q, ldc), dtype=torch.bfloat16, device=xyz.device)
-            cat_lo = mk((bs, m_q, ldc), dtype=torch.bfloat16, device=xyz.device)
-        off = 0
-        z, zoffs, wxs, hstacks, hscales = hoist.z, hoist.zoffs, hoist.wxs, hoist.stacks, hoist.scales
-        for i in range(nscale):
-            idx, cnt = idx_list[i], cnt_list[i]
-            nl = len(mlp_list[i])
-            stack = stacks[i]
-            if stack is not None:                                              # whole scale in one kernel
-                fkw = dict(out_f32=(concat, off), out_split=(cat_hi, cat_lo, off) if split_in_epilogue else None,
-                           units=units_list[i] if use_units[i] else None)
-                if hstacks.get(i) is not None:
-                    t = hscales.index(i)
-                    tf_ops.sa_mlp_fused_hoisted(xyz, z, zoffs[t], wxs[t], new_xyz, idx, cnt, hstacks[i], **fkw)
-                else:
-                    tf_ops.sa_mlp_fused(xyz, points, new_xyz, idx, cnt, stack, **fkw)
-                off += mlp_list[i][-1]
-                continue
-            hi = lo = None
-            for j in range(nl):
-                f = pp.conv("%s/conv%d_%d" % (scope, i, j), bn)
-                last_kw = dict(pool=nsample_list[i], rowmask=cnt, out_f32=(concat, off),
-                               out_split=(cat_hi, cat_lo, off) if split_in_epilogue else None)   # :167-180 conv+BN+ReLU+max+mask
-                ukw = {}
-                if use_units[i]:                  # compact rows; the last conv pools 8-row units into the zero-filled concat
-                    ukw = dict(units=units_list[i])
-                    last_kw = dict(out_f32=(concat, off), units=units_list[i], unit_pool=True)
-                if i in hscales:
-                    if j == 0:
-                        continue                  # folded into z and into the next conv's operand producer
-                    if j == 1:
-                        t = hscales.index(i)
-                        if f.kp >= HOIST_EXPAND_MIN_K and zoffs[t] % 4 == 0 and z.shape[2] % 4 == 0:
-                            # wide layer: materialise the operand once (elementwise, memory speed), plain TMA-fed GEMM
-                            hi, lo = tf_ops.hoist_expand_split(xyz, z, zoffs[t], wxs[t], new_xyz, idx, **ukw)
-                            if nl == 2:
-                                tf_ops.linear_tc(hi, lo, f, **last_kw)
-                            else:
-                                _, (hi, lo) = tf_ops.linear_tc(hi, lo, f, want_f32=False, want_split=True, **ukw)
-                            continue
-                        if nl == 2:
-                            tf_ops.linear_tc_hoisted(xyz, z, zoffs[t], wxs[t], new_xyz, idx, f, want_split=False, **last_kw)
-                        else:
-                            _, (hi, lo) = tf_ops.linear_tc_hoisted(xyz, z, zoffs[t], wxs[t], new_xyz, idx, f, **ukw)
-                        continue
-                if j == 0 and gather_in_kernel:   # :160-165 inside the kernel's operand load (no [B,M,K,C] tensor)
-                    if nl == 1:
-                        tf_ops.linear_tc_gather(xyz, points, new_xyz, idx, f, want_split=False, **last_kw)
-                    else:
-                        _, (hi, lo) = tf_ops.linear_tc_gather(xyz, points, new_xyz, idx, f)
-                    continue
-                if j == 0:                        # :160-165 fused with the split, materialised once in bf16 hi/lo
-                    hi, lo = tf_ops.group_concat_split(xyz, points, new_xyz, idx)
-                if j < nl - 1:
-                    _, (hi, lo) = tf_ops.linear_tc(hi, lo, f, want_f32=False, want_split=True, **ukw)
-                else:
-                    tf_ops.linear_tc(hi, lo, f, **last_kw)
-            off += mlp_list[i][-1]
-        new_points = concat
-        if use_agg:                                                            # :183-185
-            if not split_in_epilogue:
-                cat_hi, cat_lo = tf_ops.split_rows(concat)
-            new_points, _ = tf_ops.linear_tc(cat_hi, cat_lo, pp.conv(scope + "/ensemble", bn))
-        return new_points
-    outs = []
-    for i in range(nscale):
-        idx, cnt = idx_list[i], cnt_list[i]
-        # rows with cnt == 0 come back zero-filled, which is what idx * (cnt > 0) produces (:157-159)
-        g = tf_ops.group_concat(xyz, points, new_xyz, idx)                    # :160-165 fused
-        nl = len(mlp_list[i])
-        for j in range(nl):
-            lastl = j == nl - 1
-            g = _conv(pp, "%s/conv%d_%d" % (scope, i, j), g, bn=bn,
-                      pool=nsample_list[i] if lastl else 1, rowmask=cnt if lastl else None)   # :167-180
-        outs.append(g)
-    new_points = outs[0] if len(outs) == 1 else torch.cat(outs, dim=-1)
-    if use_agg:
-        new_points = _conv(pp, scope + "/ensemble", new_points, bn=bn)        # :183-185
-    return new_points
+        tf_ops.sa_mlp_fused(xyz, points, new_xyz, idx, cnt, s.stack, out_f32=out_f32, out_split=out_split, units=units)
 
 
-def pointnet_sa_module_msg(xyz, points, radius_list, nsample_list, mlp_list, is_training, bn_decay, bn,
-                           fps_sample_range_list, fps_method_list, npoint_list, former_fps_idx, use_attention, scope,
-                           dilated_group, vote_ctr=None, aggregation_channel=None, debugging=False, epsilon=1e-5, *,
-                           params, ffps_mode="direct", aggregation=None, return_debug=False, mlp_mode="tc",
-                           fuse_scale=True, gather_in_kernel=True, hoist_first=2, fps_cluster=0, fps_parts=None,
-                           fps_packet=False, fps_bucket=None):
-    """PointNet++ SA module with multi-scale grouping; returns (new_xyz, new_points, fps_idx).
+def _layered_scale(s, xyz, points, z, zx, new_xyz, idx, last_kw, ukw):
+    """A scale conv by conv on the tensor cores: activations stay split bf16 between the convs, the last one pools into
+    the concat buffers (last_kw); ukw carries the unit list of the compact rows."""
+    convs = list(s.convs)
+    if s.first in ("gather", "hoisted"):          # the first conv builds its operand inside the kernel (no [B,M,K,C] tensor)
+        run, args = ((tf_ops.linear_tc_hoisted, (xyz, z, *zx, new_xyz, idx)) if s.first == "hoisted"
+                     else (tf_ops.linear_tc_gather, (xyz, points, new_xyz, idx)))        # :160-165 in the operand load
+        if len(convs) == 1:
+            run(*args, convs[0], want_split=False, **last_kw)
+            return
+        _, (hi, lo) = run(*args, convs.pop(0), **ukw)
+    elif s.first == "expand":
+        hi, lo = tf_ops.hoist_expand_split(xyz, z, *zx, new_xyz, idx, **ukw)
+    else:                                         # :160-165 fused with the split, materialised once in bf16 hi/lo
+        hi, lo = tf_ops.group_concat_split(xyz, points, new_xyz, idx)
+    for f in convs[:-1]:
+        _, (hi, lo) = tf_ops.linear_tc(hi, lo, f, want_f32=False, want_split=True, **ukw)
+    tf_ops.linear_tc(hi, lo, convs[-1], **last_kw)                         # :167-180 conv+BN+ReLU+max+mask
 
-    Keyword extensions (none changes a result):
-      fps_cluster  CTAs per scene of the D-FPS kernels (tf_ops.farthest_point_sample `cluster`);
-      fps_bucket   lone D-FPS kernel choice (tf_ops.farthest_point_sample `bucket_kernel`: None automatic, False = cluster kernel);
-      fps_packet   D-FPS with the coordinates-in-packet kernel (64 KiB of shared memory per CTA instead of the whole
-                   scene: other kernels can share its SMs);
-      fps_parts    latency mode.  FPS emits its samples in order, and a sample is final once its round is done, so the
-                   layer consumes the sampling IN PARTS: a lone D-FPS runs as resumable launches of rounds (an int =
-                   that many equal parts, or a list of fractions), a fusion-sampling layer hands over its F-FPS and
-                   D-FPS halves separately; ball query + grouped MLP + aggregation of a part run on a side stream
-                   while the sampling of the next part continues, and the per-part results are joined at the end.
-                   Captured in a CUDA graph this is a plain dependency graph -- nothing polls."""
-    if use_attention:
-        raise NotImplementedError("query_ball_point_withidx (use_attention) is unused by the shipped 3DSSD configs")
-    if is_training:
-        fps_parts = None                      # training takes the literal layer-by-layer schedule
-    if mlp_mode not in ("tc", "fp32"):
-        raise ValueError("mlp_mode must be 'tc' or 'fp32'")
-    pp = prepare(params, xyz.device)
-    aggregation = _cfg.AGGREGATION_SA_FEATURE if aggregation is None else aggregation
+
+def _group_and_mlp(plan, xyz, points, z, new_xyz, radius_list, nsample_list, dilated_group):
+    """Everything of pointnet_sa_module_msg after the sampling, for one block of query points new_xyz (b, m_q, 3):
+    ball queries (:137-145), grouping + MLP + max-pool + mask per scale (:157-180), concat + aggregation (:182-185).
+    Returns (new_points, idx_list, cnt_list)."""
+    idx_list, cnt_list, units_list = _ball_query(xyz, new_xyz, radius_list, nsample_list, dilated_group,
+                                                 any(s.units for s in plan.scales))
+    if any(s.units and u is None for s, u in zip(plan.scales, units_list)):      # no unit list: those scales run dense
+        scales = [s._replace(units=s.units and u is not None) for s, u in zip(plan.scales, units_list)]
+        plan = plan._replace(scales=scales, split=plan.agg is not None and not any(s.units for s in scales))
+    if not plan.tc:
+        outs = []
+        for s, idx, cnt in zip(plan.scales, idx_list, cnt_list):
+            # rows with cnt == 0 come back zero-filled, which is what idx * (cnt > 0) produces (:157-159)
+            g = tf_ops.group_concat(xyz, points, new_xyz, idx)                 # :160-165 fused
+            for f in s.convs[:-1]:
+                g = _conv(f, g)                                                # :167-176
+            outs.append(_conv(s.convs[-1], g, pool=idx.shape[-1], rowmask=cnt))   # :167-180
+        new_points = outs[0] if len(outs) == 1 else torch.cat(outs, dim=-1)
+        return (new_points if plan.agg is None else _conv(plan.agg, new_points)), idx_list, cnt_list   # :183-185
+    # tensor cores: every scale pools straight into its slice of the concat buffer (fp32 for the caller, split bf16 for
+    # the aggregation conv).  Unit lists combine their 8-row units with atomicMax on the ZERO-FILLED fp32 buffer; the
+    # split copy the aggregation conv reads is then made once, from the finished buffer.
+    bs, m_q, _ = new_xyz.shape
+    ctot = sum(s.convs[-1].cout for s in plan.scales)
+    concat = torch.empty((bs, m_q, ctot), dtype=torch.float32, device=xyz.device)
+    if any(s.units for s in plan.scales):
+        tf_ops.fill_zero(concat)
+    cat_hi = cat_lo = None
+    if plan.split:
+        ldc = tf_ops.round16(ctot)
+        mk = torch.zeros if ldc != ctot else torch.empty
+        cat_hi, cat_lo = (mk((bs, m_q, ldc), dtype=torch.bfloat16, device=xyz.device) for _ in range(2))
+    off = 0
+    for i, s in enumerate(plan.scales):
+        idx, cnt, zx = idx_list[i], cnt_list[i], plan.hoist.get(i)
+        units = units_list[i] if s.units else None
+        out_split = (cat_hi, cat_lo, off) if plan.split else None
+        if s.stack is not None:
+            _fused_scale(s, xyz, points, z, zx, new_xyz, idx, cnt, (concat, off), out_split, units)
+        elif units is not None:                   # compact rows; the last conv pools 8-row units into the zero-filled concat
+            _layered_scale(s, xyz, points, z, zx, new_xyz, idx, dict(out_f32=(concat, off), units=units, unit_pool=True),
+                           dict(units=units))
+        else:
+            _layered_scale(s, xyz, points, z, zx, new_xyz, idx,
+                           dict(pool=idx.shape[-1], rowmask=cnt, out_f32=(concat, off), out_split=out_split), {})
+        off += s.convs[-1].cout
+    if plan.agg is None:
+        return concat, idx_list, cnt_list
+    if not plan.split:
+        cat_hi, cat_lo = tf_ops.split_rows(concat)
+    return tf_ops.linear_tc(cat_hi, cat_lo, plan.agg)[0], idx_list, cnt_list                    # :183-185
+
+
+def _sample(xyz, points, vote_ctr, fps_sample_range_list, fps_method_list, npoint_list, in_parts, fps_parts, ffps_mode,
+            fps_cluster, fps_packet, fps_bucket):
+    """The sampling of pointnet_sa_module_msg (:84-111): every segment writes its indices, segment offset included,
+    straight into fps_idx.  Returns (fps_idx, parts, nside, keep): fps_idx[:, col0:col1] is complete at `event` for each
+    (col0, col1, event) of parts (None: on the current stream), side streams 0..nside-1 ran segments, and keep holds the
+    temporaries those streams share."""
     bs, n, _ = xyz.shape
     dev = xyz.device
-    nscale = len(radius_list)
     main = torch.cuda.current_stream()
-    in_parts = bool(fps_parts) and nscale > 0 and former_fps_idx is None
-    keep = []                                  # temporaries shared between streams stay alive until the final join
-
-    # ---- hoisted first convs: the feature part of conv0 of every scale, once per POINT (independent of the sampling)
-    c_feat = points.shape[-1]
-    stacks = hoist = None
-    if nscale:
-        tc_ok = mlp_mode == "tc" and all(k in (8, 16, 32, 64, 128) for k in nsample_list) and all(m[-1] % 8 == 0 for m in mlp_list)
-        stacks = [pp.fused_stack(["%s/conv%d_%d" % (scope, i, j) for j in range(len(mlp_list[i]))], bn, c_feat + 3)
-                  if (fuse_scale and tc_ok) else None for i in range(nscale)]
-        hoist = _prepare_hoist(pp, scope, mlp_list, bn, c_feat, stacks, gather_in_kernel and tc_ok, hoist_first)
-        if in_parts and hoist.scales:          # overlaps the first rounds of the sampling
-            zs = _side_stream(dev, 7)
-            zs.wait_stream(main)
-            with torch.cuda.stream(zs):
-                _compute_hoist(hoist, pp, scope, mlp_list, bn, points, stacks)
-            z_ready = torch.cuda.Event()
-            z_ready.record(zs)
-
-    # ---- sampling (:84-111): every segment writes its indices, segment offset included, straight into fps_idx
     segs, last = [], 0
     for rng, method, npoint in zip(fps_sample_range_list, fps_method_list, npoint_list):
         end = n if rng == -1 else last + rng                      # tf.slice size -1 (:86-87)
@@ -351,6 +305,7 @@ def pointnet_sa_module_msg(xyz, points, radius_list, nsample_list, mlp_list, is_
     mtot = sum(sg[4] for sg in segs)
     fps_idx = torch.empty((bs, mtot), dtype=torch.int32, device=dev)
     parts = []                                 # (col0, col1, event): fps_idx[:, col0:col1] is complete at `event`
+    keep = []                                  # temporaries shared between streams stay alive until the final join
     col, nside = 0, 0
 
     def on_side(fn):
@@ -416,10 +371,54 @@ def pointnet_sa_module_msg(xyz, points, radius_list, nsample_list, mlp_list, is_
                                          packet_kernel=fps_packet, bucket_kernel=fps_bucket)
             parts.append((col, col + npoint, ev_main() if in_parts else None))
         col += width
+    return fps_idx, parts, nside, keep
 
-    src_xyz = vote_ctr if vote_ctr is not None else xyz
+
+def pointnet_sa_module_msg(xyz, points, radius_list, nsample_list, mlp_list, is_training, bn_decay, bn,
+                           fps_sample_range_list, fps_method_list, npoint_list, former_fps_idx, use_attention, scope,
+                           dilated_group, vote_ctr=None, aggregation_channel=None, debugging=False, epsilon=1e-5, *,
+                           params, ffps_mode="direct", aggregation=None, return_debug=False, mlp_mode="tc",
+                           fuse_scale=True, gather_in_kernel=True, hoist_first=2, fps_cluster=0, fps_parts=None,
+                           fps_packet=False, fps_bucket=None):
+    """PointNet++ SA module with multi-scale grouping; returns (new_xyz, new_points, fps_idx).
+
+    Keyword extensions (none changes a result):
+      fps_cluster  CTAs per scene of the D-FPS kernels (tf_ops.farthest_point_sample `cluster`);
+      fps_bucket   lone D-FPS kernel choice (tf_ops.farthest_point_sample `bucket_kernel`: None automatic, False = cluster kernel);
+      fps_packet   D-FPS with the coordinates-in-packet kernel (64 KiB of shared memory per CTA instead of the whole
+                   scene: other kernels can share its SMs);
+      fps_parts    latency mode.  FPS emits its samples in order, and a sample is final once its round is done, so the
+                   layer consumes the sampling IN PARTS: a lone D-FPS runs as resumable launches of rounds (an int =
+                   that many equal parts, or a list of fractions), a fusion-sampling layer hands over its F-FPS and
+                   D-FPS halves separately; ball query + grouped MLP + aggregation of a part run on a side stream
+                   while the sampling of the next part continues, and the per-part results are joined at the end.
+                   Captured in a CUDA graph this is a plain dependency graph -- nothing polls."""
+    if use_attention:
+        raise NotImplementedError("query_ball_point_withidx (use_attention) is unused by the shipped 3DSSD configs")
+    if is_training:
+        fps_parts = None                      # training takes the literal layer-by-layer schedule
+    if mlp_mode not in ("tc", "fp32"):
+        raise ValueError("mlp_mode must be 'tc' or 'fp32'")
+    pp = prepare(params, xyz.device)
+    aggregation = _cfg.AGGREGATION_SA_FEATURE if aggregation is None else aggregation
     use_agg = bool(aggregation and aggregation_channel is not None and aggregation_channel != -1)
-    debug = {"idx": [], "cnt": []}
+    dev = xyz.device
+    nscale = len(radius_list)
+    main = torch.cuda.current_stream()
+    in_parts = bool(fps_parts) and nscale > 0 and former_fps_idx is None
+    plan = _plan(pp, scope, mlp_list, nsample_list, bn, points.shape[-1], use_agg, mlp_mode, fuse_scale, gather_in_kernel,
+                 hoist_first) if (nscale and not is_training) else None
+    z = None
+    if in_parts and plan.hoist:                # the hoisted first convs overlap the first rounds of the sampling
+        zs = _side_stream(dev, 7)
+        zs.wait_stream(main)
+        with torch.cuda.stream(zs):
+            z = _hoist_table(plan, points)
+        z_ready = torch.cuda.Event()
+        z_ready.record(zs)
+    fps_idx, parts, nside, keep = _sample(xyz, points, vote_ctr, fps_sample_range_list, fps_method_list, npoint_list, in_parts,
+                                          fps_parts, ffps_mode, fps_cluster, fps_packet, fps_bucket)
+    src_xyz = vote_ctr if vote_ctr is not None else xyz
 
     if not in_parts:
         for _, _, ev in parts:
@@ -428,32 +427,30 @@ def pointnet_sa_module_msg(xyz, points, radius_list, nsample_list, mlp_list, is_
         if former_fps_idx is not None:
             fps_idx = torch.cat([fps_idx, former_fps_idx], dim=-1).contiguous()    # :113-114
         new_xyz = tf_ops.gather_point(src_xyz, fps_idx)                            # :116-119
+        debug = {"idx": [], "cnt": []}
         if nscale and is_training:
-            new_points = _group_and_mlp_train(pp, scope, xyz, points, new_xyz, radius_list, nsample_list, mlp_list, bn,
-                                              bn_decay, dilated_group, use_agg, debug)
-            debug = {"idx": debug["idx"][0], "cnt": debug["cnt"][0]}
+            new_points, debug["idx"], debug["cnt"] = _group_and_mlp_train(
+                pp, scope, xyz, points, new_xyz, radius_list, nsample_list, mlp_list, bn, bn_decay, dilated_group, use_agg)
         elif nscale:
-            _compute_hoist(hoist, pp, scope, mlp_list, bn, points, stacks)
-            new_points = _group_and_mlp(pp, scope, xyz, points, new_xyz, radius_list, nsample_list, mlp_list, bn,
-                                        dilated_group, use_agg, mlp_mode, stacks, hoist, gather_in_kernel, debug)
-            debug = {"idx": debug["idx"][0], "cnt": debug["cnt"][0]}
+            z = _hoist_table(plan, points) if plan.hoist else None
+            new_points, debug["idx"], debug["cnt"] = _group_and_mlp(plan, xyz, points, z, new_xyz, radius_list, nsample_list,
+                                                                    dilated_group)
         else:
             new_points = tf_ops.gather_point(points.contiguous(), fps_idx)         # :186-187
     else:
         # ---- one consumer chain per part, each on its own stream, joined at the end
-        xyz_parts, pts_parts, done = [], [], []
+        xyz_parts, pts_parts, nbrs, done = [], [], [], []
         for pi, (c0, c1, ev) in enumerate(parts):
             st = _side_stream(dev, 8 + pi)
             st.wait_event(ev)
-            if hoist.scales:
+            if z is not None:
                 st.wait_event(z_ready)
             with torch.cuda.stream(st):
                 nx = tf_ops.gather_point(src_xyz, fps_idx[:, c0:c1])
-                npnts = _group_and_mlp(pp, scope, xyz, points, nx, radius_list, nsample_list, mlp_list, bn, dilated_group,
-                                       use_agg, mlp_mode, stacks, hoist, gather_in_kernel, debug)
+                npnts, idx_list, cnt_list = _group_and_mlp(plan, xyz, points, z, nx, radius_list, nsample_list, dilated_group)
                 e2 = torch.cuda.Event()
                 e2.record(st)
-            xyz_parts.append(nx); pts_parts.append(npnts); done.append(e2)
+            xyz_parts.append(nx); pts_parts.append(npnts); nbrs.append((idx_list, cnt_list)); done.append(e2)
         for e2 in done:
             main.wait_event(e2)
         for i in range(nside):
@@ -461,10 +458,11 @@ def pointnet_sa_module_msg(xyz, points, radius_list, nsample_list, mlp_list, is_
         new_xyz = tf_ops.concat_rows(xyz_parts)
         new_points = tf_ops.concat_rows(pts_parts)
         keep.extend(xyz_parts + pts_parts)
+        debug = None
         if return_debug:
-            debug = {"idx": [torch.cat([d[i] for d in debug["idx"]], dim=1) for i in range(nscale)],
-                     "cnt": [torch.cat([d[i] for d in debug["cnt"]], dim=1) for i in range(nscale)]}
-        _KEEPALIVE.append((keep, debug if not return_debug else None, hoist))
+            debug = {"idx": [torch.cat([p[0][i] for p in nbrs], dim=1) for i in range(nscale)],
+                     "cnt": [torch.cat([p[1][i] for p in nbrs], dim=1) for i in range(nscale)]}
+        _KEEPALIVE.append((keep, None if return_debug else nbrs, z))
         del _KEEPALIVE[:-8]
     if return_debug:
         return new_xyz, new_points, fps_idx, debug
@@ -480,7 +478,7 @@ def pointnet_sa_module(xyz, points, mlp, is_training, bn_decay, bn, scope, *, pa
     g = torch.cat([xyz, points], dim=-1).contiguous()              # xyz FIRST here (:42)
     n = g.shape[1]
     for j in range(len(mlp)):
-        g = _conv_train(pp, "%s/conv%d" % (scope, j), g, bn, bn_decay) if is_training else _conv(pp, "%s/conv%d" % (scope, j), g, bn=bn)
+        g = _conv_train(pp, "%s/conv%d" % (scope, j), g, bn, bn_decay) if is_training else _conv(pp.conv("%s/conv%d" % (scope, j), bn), g)
     return g.max(dim=1).values if n else g
 
 
@@ -495,7 +493,7 @@ def pointnet_fp_module(xyz1, xyz2, points1, points2, mlp, is_training, bn_decay,
     if points1 is not None:
         x = torch.cat([x, points1], dim=2).contiguous()            # :213-214
     for i in range(len(mlp)):
-        x = _conv_train(pp, "%s/conv_%d" % (scope, i), x, bn, bn_decay) if is_training else _conv(pp, "%s/conv_%d" % (scope, i), x, bn=bn)
+        x = _conv_train(pp, "%s/conv_%d" % (scope, i), x, bn, bn_decay) if is_training else _conv(pp.conv("%s/conv_%d" % (scope, i), bn), x)
     return x
 
 
@@ -514,6 +512,6 @@ def vote_layer(xyz, points, mlp_list, is_training, bn_decay, bn, scope, *, param
         off, _ = tf_ops.linear_tc(hi, lo, pp.conv(scope + "/vote_offsets", False), relu=False)
     else:
         for i in range(len(mlp_list)):
-            points = _conv(pp, "%s/vote_layer_%d" % (scope, i), points, bn=bn)
-        off = _conv(pp, scope + "/vote_offsets", points, bn=False, relu=False)
+            points = _conv(pp.conv("%s/vote_layer_%d" % (scope, i), bn), points)
+        off = _conv(pp.conv(scope + "/vote_offsets", False), points, relu=False)
     return tf_ops.vote_translate(xyz, off, max_translate_range), points, off                       # :20-23

@@ -108,6 +108,9 @@ class FoldedConv:
         self.b_hi = wt.to(torch.bfloat16)                       # round-to-nearest-even, like the device split
         self.b_lo = (wt - self.b_hi.to(torch.float32)).to(torch.bfloat16)
 
+    def __repr__(self):
+        return "FoldedConv(%d -> %d)" % (self.cin, self.cout)
+
 
 def fold(params, scope, bn, device):
     """inv = gamma * rsqrt(var + eps);  y = (xW + b) * inv + (beta - mean * inv)   (tf_util.py:439-444)."""
@@ -198,6 +201,9 @@ class FusedStack:
             kp = npad
         self.w_blob = torch.cat(wparts).contiguous()
         self.ss_blob = torch.cat(sparts).contiguous()
+
+    def __repr__(self):
+        return "FusedStack(%d -> %s)" % (self.cin, self.nout)
 
 
 class PreparedParams:

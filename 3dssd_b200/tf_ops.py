@@ -25,7 +25,7 @@ def _p(t):
     return ctypes.c_void_p(t.data_ptr()) if t is not None else ctypes.c_void_p(0)
 
 
-def _req(t, name, dtype, rank, last=None):
+def _req(t, name, dtype, rank, last=None, contiguous=True):
     if not isinstance(t, torch.Tensor):
         raise ValueError("%s must be a torch.Tensor" % name)
     if not t.is_cuda:
@@ -36,22 +36,13 @@ def _req(t, name, dtype, rank, last=None):
         raise ValueError("%s must have rank %d, got shape %s" % (name, rank, tuple(t.shape)))
     if last is not None and t.shape[-1] != last:
         raise ValueError("%s must have last dimension %d, got shape %s" % (name, last, tuple(t.shape)))
-    return t if t.is_contiguous() else t.contiguous()
+    return t if (t.is_contiguous() or not contiguous) else t.contiguous()
 
 
 def _scene_strided(t, name, rank=3, last=None):
     """A float32 CUDA tensor (b, n, c) whose rows are dense but whose scenes may be strided (a [:, a:b] slice of a
     dense tensor): returns (tensor, scene stride in floats) without copying; anything else is made contiguous."""
-    if not isinstance(t, torch.Tensor):
-        raise ValueError("%s must be a torch.Tensor" % name)
-    if not t.is_cuda:
-        raise ValueError("%s must be a CUDA tensor (there is no CPU path)" % name)
-    if t.dtype != torch.float32:
-        raise ValueError("%s must be %s, got %s" % (name, torch.float32, t.dtype))
-    if t.dim() != rank:
-        raise ValueError("%s must have rank %d, got shape %s" % (name, rank, tuple(t.shape)))
-    if last is not None and t.shape[-1] != last:
-        raise ValueError("%s must have last dimension %d, got shape %s" % (name, last, tuple(t.shape)))
+    t = _req(t, name, torch.float32, rank, last, contiguous=False)
     b, n, c = t.shape
     if c > 0 and n > 0 and t.stride(2) == 1 and t.stride(1) == c and (b <= 1 or t.stride(0) >= n * c):
         return t, (t.stride(0) if b > 1 else n * c)
@@ -224,43 +215,38 @@ def _bq_shapes(xyz1, xyz2):
     return xyz1, xyz2
 
 
-def query_ball_point(radius, nsample, xyz1, xyz2):
-    """xyz1 (batch, ndataset, 3), xyz2 (batch, npoint, 3) -> idx (batch, npoint, nsample) int32,
-    pts_cnt (batch, npoint) int32.  tf_grouping.py:53-65."""
+def _query_ball(min_radius, max_radius, nsample, xyz1, xyz2, dilated):
     xyz1, xyz2 = _bq_shapes(xyz1, xyz2)
-    if not radius > 0:
-        raise ValueError("QueryBallPoint expects positive radius")      # tf_grouping.cpp:275
+    op = "QueryBallPointDilated" if dilated else "QueryBallPoint"
+    if not max_radius > 0:
+        raise ValueError("%s expects positive radius" % op)              # tf_grouping.cpp:275
     if not int(nsample) > 0:
-        raise ValueError("QueryBallPoint expects positive nsample")     # tf_grouping.cpp:278
+        raise ValueError("%s expects positive nsample" % op)             # tf_grouping.cpp:278
     b, n, _ = xyz1.shape
     m = xyz2.shape[1]
     if n >= BQ_GRID_MIN_N and lib().ssd3d_query_ball_point_workspace(b, n):
-        i, c = query_ball_point_multi([0.0], [radius], [nsample], xyz1, xyz2, False)
+        i, c = query_ball_point_multi([min_radius], [max_radius], [nsample], xyz1, xyz2, dilated)
         return i[0], c[0]
     idx = torch.empty((b, m, int(nsample)), dtype=torch.int32, device=xyz1.device)
     cnt = torch.empty((b, m), dtype=torch.int32, device=xyz1.device)
-    check(lib().ssd3d_query_ball_point(b, n, m, float(radius), int(nsample), _p(xyz1), _p(xyz2), _p(idx), _p(cnt),
-                                       _stream()), "query_ball_point")
+    io = (_p(xyz1), _p(xyz2), _p(idx), _p(cnt), _stream())
+    if dilated:
+        check(lib().ssd3d_query_ball_point_dilated(b, n, m, float(min_radius), float(max_radius), int(nsample), *io),
+              "query_ball_point_dilated")
+    else:
+        check(lib().ssd3d_query_ball_point(b, n, m, float(max_radius), int(nsample), *io), "query_ball_point")
     return idx, cnt
+
+
+def query_ball_point(radius, nsample, xyz1, xyz2):
+    """xyz1 (batch, ndataset, 3), xyz2 (batch, npoint, 3) -> idx (batch, npoint, nsample) int32,
+    pts_cnt (batch, npoint) int32.  tf_grouping.py:53-65."""
+    return _query_ball(0.0, radius, nsample, xyz1, xyz2, False)
 
 
 def query_ball_point_dilated(min_radius, max_radius, nsample, xyz1, xyz2):
     """Shell query  d == 0 or min_radius <= d < max_radius.  tf_grouping.py:68-81."""
-    xyz1, xyz2 = _bq_shapes(xyz1, xyz2)
-    if not max_radius > 0:
-        raise ValueError("QueryBallPointDilated expects positive radius")
-    if not int(nsample) > 0:
-        raise ValueError("QueryBallPointDilated expects positive nsample")
-    b, n, _ = xyz1.shape
-    m = xyz2.shape[1]
-    if n >= BQ_GRID_MIN_N and lib().ssd3d_query_ball_point_workspace(b, n):
-        i, c = query_ball_point_multi([min_radius], [max_radius], [nsample], xyz1, xyz2, True)
-        return i[0], c[0]
-    idx = torch.empty((b, m, int(nsample)), dtype=torch.int32, device=xyz1.device)
-    cnt = torch.empty((b, m), dtype=torch.int32, device=xyz1.device)
-    check(lib().ssd3d_query_ball_point_dilated(b, n, m, float(min_radius), float(max_radius), int(nsample), _p(xyz1),
-                                               _p(xyz2), _p(idx), _p(cnt), _stream()), "query_ball_point_dilated")
-    return idx, cnt
+    return _query_ball(min_radius, max_radius, nsample, xyz1, xyz2, True)
 
 
 BQ_GRID_MIN_N = 2048     # candidate sets at least this large take the spatially culled kernel (csrc/ball_query_grid.cu)
@@ -429,17 +415,24 @@ def calc_square_dist(a):
     return out
 
 
-def group_concat(xyz, points, new_xyz, idx, ldx=None):
-    """concat[group_point(points, idx), group_point(xyz, idx) - new_xyz] (layers_util.py:160-165) in one kernel.
-    Returns x (b, m, nsample, ldx) with zero padding beyond c+3."""
+def _grouping(xyz, points, new_xyz, idx):
+    """Checks of the grouping inputs xyz (b, n, 3), points (b, n, c) or None, new_xyz (b, m, 3), idx (b, m, nsample)
+    -> (xyz, points, new_xyz, idx, c)."""
     xyz = _req(xyz, "xyz", torch.float32, 3, 3)
     new_xyz = _req(new_xyz, "new_xyz", torch.float32, 3, 3)
     idx = _req(idx, "idx", torch.int32, 3)
-    b, n, _ = xyz.shape
     c = 0
     if points is not None:
         points = _req(points, "points", torch.float32, 3)
         c = points.shape[2]
+    return xyz, points, new_xyz, idx, c
+
+
+def group_concat(xyz, points, new_xyz, idx, ldx=None):
+    """concat[group_point(points, idx), group_point(xyz, idx) - new_xyz] (layers_util.py:160-165) in one kernel.
+    Returns x (b, m, nsample, ldx) with zero padding beyond c+3."""
+    xyz, points, new_xyz, idx, c = _grouping(xyz, points, new_xyz, idx)
+    b, n, _ = xyz.shape
     _, m, ns = idx.shape
     ldx = c + 3 if ldx is None else int(ldx)
     x = torch.empty((b, m, ns, ldx), dtype=torch.float32, device=xyz.device)
@@ -502,14 +495,8 @@ def split_rows(x, kp=None):
 
 def group_concat_split(xyz, points, new_xyz, idx, kp=None):
     """group_concat + split in one kernel: (hi, lo) bf16 (b, m, nsample, kp)."""
-    xyz = _req(xyz, "xyz", torch.float32, 3, 3)
-    new_xyz = _req(new_xyz, "new_xyz", torch.float32, 3, 3)
-    idx = _req(idx, "idx", torch.int32, 3)
+    xyz, points, new_xyz, idx, c = _grouping(xyz, points, new_xyz, idx)
     b, n, _ = xyz.shape
-    c = 0
-    if points is not None:
-        points = _req(points, "points", torch.float32, 3)
-        c = points.shape[2]
     _, m, ns = idx.shape
     kp = round16(c + 3) if kp is None else int(kp)
     hi = torch.empty((b, m, ns, kp), dtype=torch.bfloat16, device=xyz.device)
@@ -519,37 +506,29 @@ def group_concat_split(xyz, points, new_xyz, idx, kp=None):
     return hi, lo
 
 
-def _tc_outputs(lead, n, pool, dev, want_f32, want_split, out_f32, out_split):
-    """Resolve the output arguments shared by linear_tc / linear_tc_gather -> (y, pf, ldf, sp, ph, pl, lds)."""
-    y = None
-    pf, ldf = 0, 0
-    if out_f32 is not None:
-        buf, off = out_f32
-        ldf = buf.shape[-1]
-        pf = buf.data_ptr() + 4 * off
-        y = buf
-    elif want_f32:
-        y = torch.empty(lead + (n,), dtype=torch.float32, device=dev)
-        pf, ldf = y.data_ptr(), n
-    sp = None
-    ph = pl = 0
-    lds = 0
-    if out_split is not None:
-        hb, lb, off = out_split
-        lds = hb.shape[-1]
-        ph, pl = hb.data_ptr() + 2 * off, lb.data_ptr() + 2 * off
-        sp = (hb, lb)
-    elif want_split:
-        lds = round16(n)
-        alloc = torch.zeros if (pool > 1 and lds != n) else torch.empty
-        hb = alloc(lead + (lds,), dtype=torch.bfloat16, device=dev)
-        lb = alloc(lead + (lds,), dtype=torch.bfloat16, device=dev)
-        ph, pl = hb.data_ptr(), lb.data_ptr()
-        sp = (hb, lb)
-    return y, pf, ldf, sp, ph, pl, lds
+def _hoisted(z, zoff, wx, b, n, aligned=False):
+    """Checks of the hoisted inputs: z (b, n, ldz) fp32 holding this scale's n1 columns from zoff, wx (3, n1); aligned:
+    ldz and zoff multiples of 4.  Returns (z, (pointer to column zoff, ldz), wx, n1)."""
+    z = _req(z, "z", torch.float32, 3)
+    wx = _req(wx, "wx", torch.float32, 2)
+    n1 = wx.shape[1]
+    if (z.shape[:2] != (b, n) or wx.shape[0] != 3 or zoff < 0 or zoff + n1 > z.shape[2]
+            or (aligned and (zoff % 4 or z.shape[2] % 4))):
+        raise ValueError("z must be (b, n, ldz) with zoff + n1 <= ldz%s, and wx (3, n1)" % (", ldz and zoff multiples of 4" * aligned))
+    return z, (ctypes.c_void_p(z.data_ptr() + 4 * zoff), z.shape[2]), wx, n1
 
 
-def _tc_units_check(units, unit_pool, pool, rowmask, relu, out_f32, out_split, want_split):
+def _pooled(pool, lead):
+    """A pool width over rows of leading shape (..., nsample) -> (pool, leading shape of the outputs)."""
+    pool = int(pool)
+    if pool > 1 and (lead[-1] != pool or pool not in (8, 16, 32, 64, 128)):
+        raise ValueError("pool must equal nsample (the second-to-last dimension) and be one of 8, 16, 32, 64, 128")
+    return pool, (lead[:-1] if pool > 1 else lead)
+
+
+def _units_check(units, unit_pool=False, pool=1, rowmask=None, relu=True, out_f32=None, out_split=None, want_split=False):
+    """units: None, or the int32 CUDA unit list of query_ball_point_multi(return_units=True), which replaces pool / rowmask.
+    unit_pool: every listed 8-row unit is max-pooled into its group's row of out_f32 by atomicMax (a zero-filled buffer)."""
     if units is None:
         if unit_pool:
             raise ValueError("unit_pool needs a unit list")
@@ -559,7 +538,35 @@ def _tc_units_check(units, unit_pool, pool, rowmask, relu, out_f32, out_split, w
     if int(pool) != 1 or rowmask is not None:
         raise ValueError("a unit list replaces pool / rowmask (unit_pool=True pools the listed 8-row units)")
     if unit_pool and (not relu or out_f32 is None or out_split is not None or want_split):
-        raise ValueError("unit_pool needs relu, out_f32=(zero-filled buffer, col_offset) and no split output")
+        raise ValueError("pooling 8-row units needs relu, out_f32=(zero-filled buffer, col_offset) and no split output")
+
+
+def _tc_outputs(lead, n, pool, dev, want_f32, want_split, out_f32, out_split):
+    """Output placement of the tensor-core kernels -> (y, (hi, lo), C arguments (f32 ptr, ldf, hi ptr, lo ptr, lds)).
+    out_f32=(buffer, col) / out_split=(hi, lo, col) write into column slices of the caller's buffers, otherwise want_f32 /
+    want_split allocate lead + (n,) results (split ones padded to 16 columns, zero-filled when pooled)."""
+    y, pf, ldf = None, 0, 0
+    if out_f32 is not None:
+        y, off = out_f32
+        pf, ldf = y.data_ptr() + 4 * off, y.shape[-1]
+    elif want_f32:
+        y = torch.empty(lead + (n,), dtype=torch.float32, device=dev)
+        pf, ldf = y.data_ptr(), n
+    sp, ph, pl, lds = None, 0, 0, 0
+    if out_split is not None:
+        hb, lb, off = out_split
+        sp, ph, pl, lds = (hb, lb), hb.data_ptr() + 2 * off, lb.data_ptr() + 2 * off, hb.shape[-1]
+    elif want_split:
+        lds = round16(n)
+        alloc = torch.zeros if (pool > 1 and lds != n) else torch.empty
+        sp = tuple(alloc(lead + (lds,), dtype=torch.bfloat16, device=dev) for _ in range(2))
+        ph, pl = sp[0].data_ptr(), sp[1].data_ptr()
+    vp = ctypes.c_void_p
+    return y, sp, (vp(pf), ldf, vp(ph), vp(pl), lds)
+
+
+def _layer(f, relu):
+    return _p(f.b_hi), _p(f.b_lo), _p(f.scale), _p(f.shift), 1 if relu else 0
 
 
 def linear_tc(a_hi, a_lo, f, relu=True, pool=1, rowmask=None, want_f32=True, want_split=False, out_f32=None,
@@ -570,30 +577,20 @@ def linear_tc(a_hi, a_lo, f, relu=True, pool=1, rowmask=None, want_f32=True, wan
     units: the operand holds COMPACT rows (8 per listed unit, include/ssd3d.h ssd3d_linear_tc_units) in its first
     units[0] * 8 rows; outputs are compact likewise, or -- unit_pool=True, the last conv of a scale -- every unit is
     max-pooled and combined into out_f32[group] by atomicMax (buffer zero-filled by the caller)."""
-    _tc_units_check(units, unit_pool, pool, rowmask, relu, out_f32, out_split, want_split)
+    _units_check(units, unit_pool, pool, rowmask, relu, out_f32, out_split, want_split)
     if a_hi.dtype != torch.bfloat16 or a_lo.dtype != torch.bfloat16 or a_hi.shape != a_lo.shape:
         raise ValueError("a_hi / a_lo must be bfloat16 tensors of the same shape")
     kp = a_hi.shape[-1]
     if kp != f.kp:
         raise ValueError("operand K (%d) does not match the layer's padded K (%d)" % (kp, f.kp))
     rows = a_hi.numel() // kp
-    pool = int(pool)
-    lead = tuple(a_hi.shape[:-1])
-    if pool > 1:
-        if lead[-1] != pool or pool not in (8, 16, 32, 64, 128):
-            raise ValueError("pool must equal the second-to-last dimension and be one of 8, 16, 32, 64, 128")
-        lead = lead[:-1]
-    n = f.cout
-    y, pf, ldf, sp, ph, pl, lds = _tc_outputs(lead, n, pool, a_hi.device, want_f32, want_split, out_f32, out_split)
-    vp = ctypes.c_void_p
+    pool, lead = _pooled(pool, tuple(a_hi.shape[:-1]))
+    y, sp, io = _tc_outputs(lead, f.cout, pool, a_hi.device, want_f32, want_split, out_f32, out_split)
+    a = (rows, kp, f.cout, _p(a_hi), _p(a_lo)) + _layer(f, relu)
     if units is not None:
-        check(lib().ssd3d_linear_tc_units(rows, kp, n, _p(a_hi), _p(a_lo), _p(f.b_hi), _p(f.b_lo), _p(f.scale), _p(f.shift),
-                                          1 if relu else 0, _p(units), 1 if unit_pool else 0, vp(pf), ldf, vp(ph), vp(pl), lds,
-                                          _stream()), "linear_tc_units")
-        return y, sp
-    check(lib().ssd3d_linear_tc(rows, kp, n, _p(a_hi), _p(a_lo), _p(f.b_hi), _p(f.b_lo), _p(f.scale), _p(f.shift),
-                                1 if relu else 0, pool, _p(rowmask), vp(pf), ldf, vp(ph), vp(pl), lds, _stream()),
-          "linear_tc")
+        check(lib().ssd3d_linear_tc_units(*a, _p(units), 1 if unit_pool else 0, *io, _stream()), "linear_tc_units")
+    else:
+        check(lib().ssd3d_linear_tc(*a, pool, _p(rowmask), *io, _stream()), "linear_tc")
     return y, sp
 
 
@@ -602,26 +599,15 @@ def linear_tc_gather(xyz, points, new_xyz, idx, f, relu=True, pool=1, rowmask=No
     """First conv layer of an SA scale with the gather / centre-subtract / concat of layers_util.py:160-165 fused
     into the tensor-core kernel's operand load (no [B,M,K,C] tensor in HBM).  Outputs as linear_tc, leading shape
     (b, m, nsample) or (b, m) when pooled."""
-    xyz = _req(xyz, "xyz", torch.float32, 3, 3)
-    new_xyz = _req(new_xyz, "new_xyz", torch.float32, 3, 3)
-    idx = _req(idx, "idx", torch.int32, 3)
-    b, n, _ = xyz.shape
-    c = 0
-    if points is not None:
-        points = _req(points, "points", torch.float32, 3)
-        c = points.shape[2]
+    xyz, points, new_xyz, idx, c = _grouping(xyz, points, new_xyz, idx)
     if round16(c + 3) != f.kp or c + 3 != f.cin:
         raise ValueError("layer input width %d does not match c+3 = %d" % (f.cin, c + 3))
+    b, n, _ = xyz.shape
     _, m, ns = idx.shape
-    pool = int(pool)
-    if pool > 1 and (pool != ns or pool not in (8, 16, 32, 64, 128)):
-        raise ValueError("pool must equal nsample and be one of 8, 16, 32, 64, 128")
-    lead = (b, m) if pool > 1 else (b, m, ns)
-    y, pf, ldf, sp, ph, pl, lds = _tc_outputs(lead, f.cout, pool, xyz.device, want_f32, want_split, out_f32, out_split)
-    vp = ctypes.c_void_p
-    check(lib().ssd3d_linear_tc_gather(b, n, c, m, ns, _p(xyz), _p(points), _p(new_xyz), _p(idx), f.cout, _p(f.b_hi),
-                                       _p(f.b_lo), _p(f.scale), _p(f.shift), 1 if relu else 0, pool, _p(rowmask), vp(pf),
-                                       ldf, vp(ph), vp(pl), lds, _stream()), "linear_tc_gather")
+    pool, lead = _pooled(pool, (b, m, ns))
+    y, sp, io = _tc_outputs(lead, f.cout, pool, xyz.device, want_f32, want_split, out_f32, out_split)
+    check(lib().ssd3d_linear_tc_gather(b, n, c, m, ns, _p(xyz), _p(points), _p(new_xyz), _p(idx), f.cout, *_layer(f, relu),
+                                       pool, _p(rowmask), *io, _stream()), "linear_tc_gather")
     return y, sp
 
 
@@ -631,34 +617,22 @@ def linear_tc_hoisted(xyz, z, zoff, wx, new_xyz, idx, f, relu=True, pool=1, rowm
     z: (b, n, ldz) fp32 per-point table = (features . Wf) * s1 + t1 for all scales of the layer, this scale's
     columns start at zoff; wx: (3, n1) fp32 = Wx * s1; f: params.FoldedConv of the second conv (cin == n1).
     units / unit_pool: as linear_tc (the source rows are looked up through the list, outputs are compact)."""
-    _tc_units_check(units, unit_pool, pool, rowmask, relu, out_f32, out_split, want_split)
-    xyz = _req(xyz, "xyz", torch.float32, 3, 3)
-    new_xyz = _req(new_xyz, "new_xyz", torch.float32, 3, 3)
-    idx = _req(idx, "idx", torch.int32, 3)
-    z = _req(z, "z", torch.float32, 3)
-    wx = _req(wx, "wx", torch.float32, 2)
+    _units_check(units, unit_pool, pool, rowmask, relu, out_f32, out_split, want_split)
+    xyz, _, new_xyz, idx, _ = _grouping(xyz, None, new_xyz, idx)
     b, n, _ = xyz.shape
-    n1 = wx.shape[1]
-    if z.shape[:2] != (b, n) or wx.shape[0] != 3 or zoff < 0 or zoff + n1 > z.shape[2]:
-        raise ValueError("z must be (b, n, ldz) with zoff + n1 <= ldz and wx (3, n1)")
+    z, zcols, wx, n1 = _hoisted(z, zoff, wx, b, n)
     if f.cin != n1:
         raise ValueError("second conv expects %d inputs, the hoisted first conv has %d outputs" % (f.cin, n1))
     _, m, ns = idx.shape
-    pool = int(pool)
-    if pool > 1 and (pool != ns or pool not in (8, 16, 32, 64, 128)):
-        raise ValueError("pool must equal nsample and be one of 8, 16, 32, 64, 128")
-    lead = (b, m) if pool > 1 else (b, m, ns)
-    y, pf, ldf, sp, ph, pl, lds = _tc_outputs(lead, f.cout, pool, xyz.device, want_f32, want_split, out_f32, out_split)
-    vp = ctypes.c_void_p
+    pool, lead = _pooled(pool, (b, m, ns))
+    y, sp, io = _tc_outputs(lead, f.cout, pool, xyz.device, want_f32, want_split, out_f32, out_split)
+    a = (b, n, n1, m, ns, _p(xyz), *zcols, _p(wx), _p(new_xyz), _p(idx))
     if units is not None:
-        check(lib().ssd3d_linear_tc_hoisted_units(b, n, n1, m, ns, _p(xyz), vp(z.data_ptr() + 4 * zoff), z.shape[2], _p(wx),
-                                                  _p(new_xyz), _p(idx), _p(units), f.cout, _p(f.b_hi), _p(f.b_lo), _p(f.scale),
-                                                  _p(f.shift), 1 if relu else 0, 1 if unit_pool else 0, vp(pf), ldf, vp(ph),
-                                                  vp(pl), lds, _stream()), "linear_tc_hoisted_units")
-        return y, sp
-    check(lib().ssd3d_linear_tc_hoisted(b, n, n1, m, ns, _p(xyz), vp(z.data_ptr() + 4 * zoff), z.shape[2], _p(wx), _p(new_xyz),
-                                        _p(idx), f.cout, _p(f.b_hi), _p(f.b_lo), _p(f.scale), _p(f.shift), 1 if relu else 0,
-                                        pool, _p(rowmask), vp(pf), ldf, vp(ph), vp(pl), lds, _stream()), "linear_tc_hoisted")
+        check(lib().ssd3d_linear_tc_hoisted_units(*a, _p(units), f.cout, *_layer(f, relu), 1 if unit_pool else 0, *io,
+                                                  _stream()), "linear_tc_hoisted_units")
+    else:
+        check(lib().ssd3d_linear_tc_hoisted(*a, f.cout, *_layer(f, relu), pool, _p(rowmask), *io, _stream()),
+              "linear_tc_hoisted")
     return y, sp
 
 
@@ -667,37 +641,26 @@ def hoist_expand_split(xyz, z, zoff, wx, new_xyz, idx, units=None):
     split(relu(z[idx] + (xyz[idx] - new_xyz) . wx)).  Followed by the plain linear_tc this is the faster route for wide
     layers (K >= 256), where the resident operand of the in-kernel route leaves the weight ring two narrow stages.
     units: only the listed 8-row units are built, as compact rows at the start of the buffers."""
-    xyz = _req(xyz, "xyz", torch.float32, 3, 3)
-    new_xyz = _req(new_xyz, "new_xyz", torch.float32, 3, 3)
-    idx = _req(idx, "idx", torch.int32, 3)
-    z = _req(z, "z", torch.float32, 3)
-    wx = _req(wx, "wx", torch.float32, 2)
+    _units_check(units)
+    xyz, _, new_xyz, idx, _ = _grouping(xyz, None, new_xyz, idx)
     b, n, _ = xyz.shape
-    n1 = wx.shape[1]
-    if z.shape[:2] != (b, n) or wx.shape[0] != 3 or zoff < 0 or zoff + n1 > z.shape[2] or zoff % 4 or z.shape[2] % 4:
-        raise ValueError("z must be (b, n, ldz) with ldz, zoff multiples of 4, zoff + n1 <= ldz, and wx (3, n1)")
+    z, zcols, wx, n1 = _hoisted(z, zoff, wx, b, n, aligned=True)
     _, m, ns = idx.shape
     kp = round16(n1)
     hi = torch.empty((b, m, ns, kp), dtype=torch.bfloat16, device=xyz.device)
     lo = torch.empty_like(hi)
+    a = (b, n, n1, m, ns, _p(xyz), *zcols, _p(wx), _p(new_xyz), _p(idx))
     if units is not None:
-        _tc_units_check(units, False, 1, None, True, None, None, False)
-        check(lib().ssd3d_hoist_expand_split_units(b, n, n1, m, ns, _p(xyz), ctypes.c_void_p(z.data_ptr() + 4 * zoff), z.shape[2],
-                                                   _p(wx), _p(new_xyz), _p(idx), _p(units), _p(hi), _p(lo), kp, _stream()),
-              "hoist_expand_split_units")
-        return hi, lo
-    check(lib().ssd3d_hoist_expand_split(b, n, n1, m, ns, _p(xyz), ctypes.c_void_p(z.data_ptr() + 4 * zoff), z.shape[2], _p(wx),
-                                         _p(new_xyz), _p(idx), _p(hi), _p(lo), kp, _stream()), "hoist_expand_split")
+        check(lib().ssd3d_hoist_expand_split_units(*a, _p(units), _p(hi), _p(lo), kp, _stream()), "hoist_expand_split_units")
+    else:
+        check(lib().ssd3d_hoist_expand_split(*a, _p(hi), _p(lo), kp, _stream()), "hoist_expand_split")
     return hi, lo
 
 
-def _units_check(units, out_f32, out_split):
-    if units is None:
-        return
-    if units.dtype != torch.int32 or not units.is_cuda or not units.is_contiguous():
-        raise ValueError("units must be the int32 CUDA unit list returned by query_ball_point_multi(return_units=True)")
-    if out_f32 is None or out_split is not None:
-        raise ValueError("a unit list needs out_f32=(zero-filled buffer, col_offset) and no out_split (results combine through atomicMax)")
+def _stack(stack):
+    nout = (ctypes.c_int * len(stack.nout))(*stack.nout)        # the cast keeps the array alive
+    return (len(stack.nout), ctypes.cast(nout, ctypes.c_void_p), _p(stack.w_blob), _p(stack.ss_blob),
+            1 if stack.last_scale_nonneg else 0)
 
 
 def sa_mlp_fused(xyz, points, new_xyz, idx, cnt, stack, out_f32=None, out_split=None, units=None):
@@ -707,74 +670,31 @@ def sa_mlp_fused(xyz, points, new_xyz, idx, cnt, stack, out_f32=None, out_split=
     units: the scale's unit list (query_ball_point_multi(return_units=True)): only the listed 8-row units are convolved
     -- the skipped rows repeat a group's first neighbour and cannot change the max-pool -- and results are combined with
     atomicMax into out_f32, which must be zero-filled (fill_zero)."""
-    _units_check(units, out_f32, out_split)
-    xyz = _req(xyz, "xyz", torch.float32, 3, 3)
-    new_xyz = _req(new_xyz, "new_xyz", torch.float32, 3, 3)
-    idx = _req(idx, "idx", torch.int32, 3)
-    b, n, _ = xyz.shape
-    c = 0
-    if points is not None:
-        points = _req(points, "points", torch.float32, 3)
-        c = points.shape[2]
+    _units_check(units, units is not None, out_f32=out_f32, out_split=out_split)
+    xyz, points, new_xyz, idx, c = _grouping(xyz, points, new_xyz, idx)
     if c + 3 != stack.cin:
         raise ValueError("feature channels (%d) do not match the stack's input width (%d)" % (c, stack.cin - 3))
+    b, n, _ = xyz.shape
     _, m, ns = idx.shape
-    n3 = stack.nout[-1]
-    y = None
-    pf, ldf = 0, 0
-    if out_f32 is not None:
-        buf, off = out_f32
-        ldf, pf, y = buf.shape[-1], buf.data_ptr() + 4 * off, buf
-    elif out_split is None:
-        y = torch.empty((b, m, n3), dtype=torch.float32, device=xyz.device)
-        pf, ldf = y.data_ptr(), n3
-    ph = pl = lds = 0
-    if out_split is not None:
-        hb, lb, off = out_split
-        lds, ph, pl = hb.shape[-1], hb.data_ptr() + 2 * off, lb.data_ptr() + 2 * off
-    nout = (ctypes.c_int * len(stack.nout))(*stack.nout)
-    vp = ctypes.c_void_p
-    check(lib().ssd3d_sa_mlp_fused(b, n, c, m, ns, _p(xyz), _p(points), _p(new_xyz), _p(idx), _p(cnt), _p(units), len(stack.nout),
-                                   ctypes.cast(nout, vp), _p(stack.w_blob), _p(stack.ss_blob), 1 if stack.last_scale_nonneg else 0,
-                                   vp(pf), ldf, vp(ph), vp(pl), lds, _stream()), "sa_mlp_fused")
+    y, _, io = _tc_outputs((b, m), stack.nout[-1], 1, xyz.device, out_split is None, False, out_f32, out_split)
+    check(lib().ssd3d_sa_mlp_fused(b, n, c, m, ns, _p(xyz), _p(points), _p(new_xyz), _p(idx), _p(cnt), _p(units),
+                                   *_stack(stack), *io, _stream()), "sa_mlp_fused")
     return y
 
 
 def sa_mlp_fused_hoisted(xyz, z, zoff, wx, new_xyz, idx, cnt, stack, out_f32=None, out_split=None, units=None):
     """sa_mlp_fused with the scale's first conv hoisted into the per-point table z (see linear_tc_hoisted): `stack` is the
     params.FusedStack of the REMAINING convs (its input width == wx.shape[1]).  units: as sa_mlp_fused."""
-    _units_check(units, out_f32, out_split)
-    xyz = _req(xyz, "xyz", torch.float32, 3, 3)
-    new_xyz = _req(new_xyz, "new_xyz", torch.float32, 3, 3)
-    idx = _req(idx, "idx", torch.int32, 3)
-    z = _req(z, "z", torch.float32, 3)
-    wx = _req(wx, "wx", torch.float32, 2)
+    _units_check(units, units is not None, out_f32=out_f32, out_split=out_split)
+    xyz, _, new_xyz, idx, _ = _grouping(xyz, None, new_xyz, idx)
     b, n, _ = xyz.shape
-    n1 = wx.shape[1]
-    if z.shape[:2] != (b, n) or wx.shape[0] != 3 or zoff < 0 or zoff + n1 > z.shape[2]:
-        raise ValueError("z must be (b, n, ldz) with zoff + n1 <= ldz and wx (3, n1)")
+    z, zcols, wx, n1 = _hoisted(z, zoff, wx, b, n)
     if n1 != stack.cin:
         raise ValueError("hoisted width (%d) does not match the stack's input width (%d)" % (n1, stack.cin))
     _, m, ns = idx.shape
-    n3 = stack.nout[-1]
-    y = None
-    pf, ldf = 0, 0
-    if out_f32 is not None:
-        buf, off = out_f32
-        ldf, pf, y = buf.shape[-1], buf.data_ptr() + 4 * off, buf
-    elif out_split is None:
-        y = torch.empty((b, m, n3), dtype=torch.float32, device=xyz.device)
-        pf, ldf = y.data_ptr(), n3
-    ph = pl = lds = 0
-    if out_split is not None:
-        hb, lb, off = out_split
-        lds, ph, pl = hb.shape[-1], hb.data_ptr() + 2 * off, lb.data_ptr() + 2 * off
-    nout = (ctypes.c_int * len(stack.nout))(*stack.nout)
-    vp = ctypes.c_void_p
-    check(lib().ssd3d_sa_mlp_fused_hoisted(b, n, n1, m, ns, _p(xyz), vp(z.data_ptr() + 4 * zoff), z.shape[2], _p(wx), _p(new_xyz),
-                                           _p(idx), _p(cnt), _p(units), len(stack.nout), ctypes.cast(nout, vp), _p(stack.w_blob),
-                                           _p(stack.ss_blob), 1 if stack.last_scale_nonneg else 0, vp(pf), ldf, vp(ph), vp(pl),
-                                           lds, _stream()), "sa_mlp_fused_hoisted")
+    y, _, io = _tc_outputs((b, m), stack.nout[-1], 1, xyz.device, out_split is None, False, out_f32, out_split)
+    check(lib().ssd3d_sa_mlp_fused_hoisted(b, n, n1, m, ns, _p(xyz), *zcols, _p(wx), _p(new_xyz), _p(idx), _p(cnt), _p(units),
+                                           *_stack(stack), *io, _stream()), "sa_mlp_fused_hoisted")
     return y
 
 

@@ -5,6 +5,9 @@ resumable rounds, the latency-mode part schedule and its joins -- runs here with
 oracle's own layer code.  (The kernels themselves are covered by the -m gpu tests.)"""
 import copy
 import importlib
+import inspect
+import json
+import os
 
 import numpy as np
 import pytest
@@ -239,10 +242,70 @@ def _scaled(pkg, div):
     return arch
 
 
+ROUTE_TRACE = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "sa_route_trace.json")
+
+
+def _record_calls(monkeypatch, pkg):
+    """Wrap every tf_ops entry point: each call the layers make is appended to the returned list as [name, positional
+    args, keyword args], tensors reduced to dtype and shape, folded convs to (cin, cout), fused stacks to their widths.
+    The sequence is the host-side launch schedule of the forward: same calls, same order, same operand shapes."""
+    T, P = pkg.tf_ops, pkg.params
+    calls = []
+
+    def enc(v):
+        if isinstance(v, torch.Tensor):
+            return "%s%s" % (str(v.dtype).replace("torch.", ""), list(v.shape))
+        if isinstance(v, P.FoldedConv):
+            return ["FoldedConv", v.cin, v.cout]
+        if isinstance(v, P.FusedStack):
+            return ["FusedStack", list(v.nout)]
+        if isinstance(v, (list, tuple)):
+            return [enc(x) for x in v]
+        if isinstance(v, torch.device):
+            return str(v.type)
+        if v is None or isinstance(v, (bool, int, float, str)):
+            return v
+        raise TypeError("no trace encoding for %r" % (v,))
+
+    for name, fn in list(vars(T).items()):
+        if name.startswith("_") or name in ("check", "lib", "round16") or not inspect.isfunction(fn):
+            continue
+
+        def rec(*a, _fn=fn, _name=name, **kw):
+            calls.append([_name, enc(a), {k: enc(kw[k]) for k in sorted(kw)}])
+            return _fn(*a, **kw)
+        monkeypatch.setattr(T, name, rec)
+    return calls
+
+
+def _check_route_trace(key, calls):
+    """Compare with the stored trace; SSD3D_WRITE_ROUTE_TRACE=1 stores this run's trace instead (a deliberate change of
+    the launch schedule)."""
+    store = {}
+    if os.path.exists(ROUTE_TRACE):
+        with open(ROUTE_TRACE) as fh:
+            store = json.load(fh)
+    got = json.loads(json.dumps(calls))
+    if os.environ.get("SSD3D_WRITE_ROUTE_TRACE"):
+        store[key] = got
+        with open(ROUTE_TRACE, "w") as fh:
+            fh.write("{\n" + ",\n".join("%s: [\n%s\n]" % (json.dumps(k), ",\n".join(json.dumps(c) for c in store[k]))
+                                        for k in sorted(store)) + "\n}\n")
+        return
+    assert key in store, "no stored route trace for %s (SSD3D_WRITE_ROUTE_TRACE=1 records it)" % key
+    exp = store[key]
+    for i, (g, e) in enumerate(zip(got, exp)):
+        assert g == e, "call %d of the route differs:\n  got      %s\n  expected %s" % (i, g, e)
+    assert len(got) == len(exp), "the route makes %d tf_ops calls, expected %d" % (len(got), len(exp))
+
+
 @pytest.mark.parametrize("mlp_mode,gather,hoist,fuse", [("fp32", True, 2, True), ("tc", True, 2, True), ("tc", True, 1, True),
                                                         ("tc", True, 0, True), ("tc", False, 0, False), ("tc", True, 2, False)])
 @pytest.mark.parametrize("latency,parts", [(False, None), (True, 2), (True, [0.5, 0.25, 0.25])])
-def test_backbone_orchestration_dry_run_matches_oracle_layers(dry, oracle_ops, latency, parts, mlp_mode, gather, hoist, fuse):
+def test_backbone_orchestration_dry_run_matches_oracle_layers(dry, oracle_ops, monkeypatch, request, latency, parts, mlp_mode,
+                                                              gather, hoist, fuse):
+    """The layer outputs equal the oracle's, and the sequence of tf_ops calls equals tests/golden/sa_route_trace.json
+    (the tc / fused / default-latency case also with layers_util.COMPACT_GROUPS off)."""
     pkg = dry
     from oracle import layers as olayers
     synth = importlib.import_module("3dssd_b200.synth")
@@ -253,16 +316,24 @@ def test_backbone_orchestration_dry_run_matches_oracle_layers(dry, oracle_ops, l
     kw = dict(fps_parts=parts) if parts is not None else {}
     net = pkg.SABackbone(arch, params, in_channels=1, device="cpu", mlp_mode=mlp_mode, latency_mode=latency,
                          gather_in_kernel=gather, hoist_first=hoist, fuse_scale=fuse, **kw)
-    got = net.forward(torch.from_numpy(pts), return_debug=True)
     exp = olayers.backbone_forward(arch, pts, params, ffps_mode="matrix", return_debug=True)
-    for li in range(1, len(arch) + 1):
-        if exp[2][li] is not None:
-            np.testing.assert_array_equal(got[2][li].numpy(), exp[2][li], err_msg="fps_idx of layer %d" % li)
-        for a, b in zip(got[3][li - 1].get("idx", []), exp[3][li - 1].get("idx", [])):
-            np.testing.assert_array_equal(a.numpy(), b)
-        if exp[0][li] is not None:
-            assert np.abs(got[0][li].numpy() - exp[0][li]).max() < 1e-5
-        assert np.abs(got[1][li].numpy() - exp[1][li]).max() <= 1e-4 * max(1.0, np.abs(exp[1][li]).max()), "features of layer %d" % li
+    calls = _record_calls(monkeypatch, pkg)
+    runs = [request.node.callspec.id]
+    if (mlp_mode, gather, hoist, fuse, latency) == ("tc", True, 2, True, False):
+        runs.append(runs[0] + "-nocompact")
+    for key in runs:
+        monkeypatch.setattr(pkg.layers_util, "COMPACT_GROUPS", not key.endswith("-nocompact"))
+        del calls[:]
+        got = net.forward(torch.from_numpy(pts), return_debug=True)
+        for li in range(1, len(arch) + 1):
+            if exp[2][li] is not None:
+                np.testing.assert_array_equal(got[2][li].numpy(), exp[2][li], err_msg="fps_idx of layer %d" % li)
+            for a, b in zip(got[3][li - 1].get("idx", []), exp[3][li - 1].get("idx", [])):
+                np.testing.assert_array_equal(a.numpy(), b)
+            if exp[0][li] is not None:
+                assert np.abs(got[0][li].numpy() - exp[0][li]).max() < 1e-5
+            assert np.abs(got[1][li].numpy() - exp[1][li]).max() <= 1e-4 * max(1.0, np.abs(exp[1][li]).max()), "features of layer %d" % li
+        _check_route_trace(key, calls)
 
 
 def test_head_orchestration_dry_run_writes_into_gather_buffers(dry, oracle_ops, monkeypatch):
