@@ -75,7 +75,7 @@ ball_query_kernel(const float *__restrict__ xyz1, const float *__restrict__ xyz2
     if (tid == 0) {
         mbar_init(smem_u32(&full_bar[0]), p.use_tma ? 1 : BQ_THREADS);
         mbar_init(smem_u32(&full_bar[1]), p.use_tma ? 1 : BQ_THREADS);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        fence_mbar_init_cluster();
     }
     __syncthreads();
 
@@ -92,7 +92,7 @@ ball_query_kernel(const float *__restrict__ xyz1, const float *__restrict__ xyz2
             }
         } else {
             for (int i = tid; i < npts * 3; i += BQ_THREADS) dst[i] = cand[(size_t)base * 3 + i];
-            asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(&full_bar[stage])) : "memory");
+            mbar_arrive(smem_u32(&full_bar[stage]));
         }
     };
 

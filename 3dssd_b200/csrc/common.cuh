@@ -61,6 +61,10 @@ __device__ __forceinline__ void fence_mbar_init_cluster()
 {
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
 }
+__device__ __forceinline__ void mbar_arrive(uint32_t bar)
+{
+    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
+}
 __device__ __forceinline__ void mbar_arrive_expect_tx(uint32_t bar, uint32_t bytes)
 {
     asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
@@ -76,6 +80,8 @@ __device__ __forceinline__ void mbar_wait_cluster(uint32_t bar, uint32_t parity)
         "DONE_%=:\n\t}"
         ::"r"(bar), "r"(parity) : "memory");
 }
+// named barrier `id` (1..15) over `nthreads` threads (a multiple of 32)
+__device__ __forceinline__ void bar_sync(int id, int nthreads) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory"); }
 // One lane of a converged warp (for single-thread instructions such as tcgen05.mma / commit issued from code the
 // whole warp runs, so that their operands stay in uniform registers).
 __device__ __forceinline__ bool elect_one()
@@ -120,5 +126,15 @@ __device__ __forceinline__ void bulk_g2s(uint32_t dst, const void *src, uint32_t
     asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
                  ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
 }
+
+
+// Order-preserving float <-> uint map: unsigned comparisons (redux.min/max, sort keys) of ord(x) order the floats x,
+// negative values included.
+__device__ __forceinline__ uint32_t f2ord(float x)
+{
+    const uint32_t b = __float_as_uint(x);
+    return (b & 0x80000000u) ? ~b : (b | 0x80000000u);
+}
+__device__ __forceinline__ float ord2f(uint32_t u) { return __uint_as_float((u & 0x80000000u) ? (u & 0x7fffffffu) : ~u); }
 
 }  // namespace ssd3d

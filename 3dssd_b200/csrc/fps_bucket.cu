@@ -41,14 +41,6 @@ constexpr int FB_NBUCKET = FB_NW * FB_SLOTS; // 512
 constexpr int FB_MAXN = FB_NBUCKET * 32;     // 16384 points
 constexpr uint32_t FB_PAD_KEY = 0xFFFFFFFFu;
 
-// order-preserving float <-> uint map for min/max reductions of signed floats
-__device__ __forceinline__ uint32_t fb_ord(float x)
-{
-    const uint32_t b = __float_as_uint(x);
-    return (b & 0x80000000u) ? ~b : (b | 0x80000000u);
-}
-__device__ __forceinline__ float fb_unord(uint32_t u) { return __uint_as_float((u & 0x80000000u) ? (u & 0x7fffffffu) : ~u); }
-
 __device__ __forceinline__ uint32_t fb_spread9(uint32_t v)   // 9 bits -> every second bit
 {
     v &= 0x1ffu;
@@ -110,7 +102,7 @@ fps3_bucket_kernel(int n, int m, const float *__restrict__ inp, int *__restrict_
         }
 #pragma unroll
         for (int a = 0; a < 3; a++) {
-            const uint32_t mn = __reduce_min_sync(0xffffffffu, fb_ord(lo[a])), mx = __reduce_max_sync(0xffffffffu, fb_ord(hi[a]));
+            const uint32_t mn = __reduce_min_sync(0xffffffffu, f2ord(lo[a])), mx = __reduce_max_sync(0xffffffffu, f2ord(hi[a]));
             if (lane == 0) { red[a][w] = mn; red[3 + a][w] = mx; }
         }
         __syncthreads();
@@ -119,7 +111,7 @@ fps3_bucket_kernel(int n, int m, const float *__restrict__ inp, int *__restrict_
         for (int a = 0; a < 3; a++) {
             uint32_t mn = 0xffffffffu, mx = 0u;
             for (int q = 0; q < FB_NW; q++) { mn = min(mn, red[a][q]); mx = max(mx, red[3 + a][q]); }
-            lo[a] = fb_unord(mn); hi[a] = fb_unord(mx);
+            lo[a] = ord2f(mn); hi[a] = ord2f(mx);
             ext[a] = hi[a] - lo[a];
         }
         // the two widest axes (a0 widest), square cells sized by the widest; non-finite extents just give poor buckets
@@ -183,20 +175,20 @@ fps3_bucket_kernel(int n, int m, const float *__restrict__ inp, int *__restrict_
         if (valid) { x = __ldg(data + 3 * o); y = __ldg(data + 3 * o + 1); z = __ldg(data + 3 * o + 2); }
         xs[p] = x; ys[p] = y; zs[p] = z;
         dist[i] = valid ? (resume ? tsave[o] : 1e38f) : -1.0f;    // tf_sampling_g.cu:136
-        const uint32_t mnx = __reduce_min_sync(0xffffffffu, valid ? fb_ord(x) : 0xffffffffu);
-        const uint32_t mny = __reduce_min_sync(0xffffffffu, valid ? fb_ord(y) : 0xffffffffu);
-        const uint32_t mnz = __reduce_min_sync(0xffffffffu, valid ? fb_ord(z) : 0xffffffffu);
-        const uint32_t mxx = __reduce_max_sync(0xffffffffu, valid ? fb_ord(x) : 0u);
-        const uint32_t mxy = __reduce_max_sync(0xffffffffu, valid ? fb_ord(y) : 0u);
-        const uint32_t mxz = __reduce_max_sync(0xffffffffu, valid ? fb_ord(z) : 0u);
+        const uint32_t mnx = __reduce_min_sync(0xffffffffu, valid ? f2ord(x) : 0xffffffffu);
+        const uint32_t mny = __reduce_min_sync(0xffffffffu, valid ? f2ord(y) : 0xffffffffu);
+        const uint32_t mnz = __reduce_min_sync(0xffffffffu, valid ? f2ord(z) : 0xffffffffu);
+        const uint32_t mxx = __reduce_max_sync(0xffffffffu, valid ? f2ord(x) : 0u);
+        const uint32_t mxy = __reduce_max_sync(0xffffffffu, valid ? f2ord(y) : 0u);
+        const uint32_t mxz = __reduce_max_sync(0xffffffffu, valid ? f2ord(z) : 0u);
         // arg-max of the slot as it stands (a fresh start has 1e38 everywhere: every bucket is "affected" in round 1)
         const uint32_t u = valid ? __float_as_uint(fmaxf(dist[i], 0.0f)) : 0u;
         const uint32_t key = valid ? fb_key(o, (uint32_t)p) : KEY_INVALID;
         uint32_t mx, kmin;
         warp_argmax(u, key, mx, kmin);
         if (lane == i) {
-            bminx = fb_unord(mnx); bminy = fb_unord(mny); bminz = fb_unord(mnz);
-            bmaxx = fb_unord(mxx); bmaxy = fb_unord(mxy); bmaxz = fb_unord(mxz);
+            bminx = ord2f(mnx); bminy = ord2f(mny); bminz = ord2f(mnz);
+            bmaxx = ord2f(mxx); bmaxy = ord2f(mxy); bmaxz = ord2f(mxz);
             bmaxu = mx; bkey = kmin;
         }
     }

@@ -7,7 +7,7 @@
 // Precision (DESIGN.md "Grouped MLP"): the reference computes in fp32 and the parity budget is 1e-3 relative.
 // A single TF32/BF16 pass does not hold that through three chained layers, so every fp32 operand is split into
 // two bf16 terms, x = x_hi + x_lo (16 mantissa bits), and the product is evaluated as three bf16 MMAs
-//     x.W ~= x_hi.W_hi + x_lo.W_hi + x_hi.W_lo          (error ~2^-16, fp32 accumulation in TMEM)
+//     x.W ~= x_hi.W_hi + x_lo.W_hi + x_hi.W_lo          (error ~2^-16, fp32 accumulation in TMEM; tc.cuh)
 // at 3x the bf16 tensor rate instead of the 2x-slower TF32 pipe.  Activations travel between layers already
 // split (two bf16 matrices, row-major == K-major), so every operand tile is a plain TMA box in the 128B-swizzled
 // canonical UMMA layout and no conversion happens on the load path.
@@ -24,14 +24,13 @@
 // Unit-list mode (TcParams::units, round 2): the grouped matrix holds only the 8-row units the ball query listed (rows
 // that repeat a group's first neighbour cannot change the max-pool); the row count comes from the list at run time, the
 // gather producers look their source up through it, and the last conv of a scale pools each unit and combines the units
-// of a group with atomicMax (pooled_units_chunk).  Same bits as the dense schedule.
-#include <cuda.h>
-#include <cuda_bf16.h>
+// of a group with atomicMax (pool_units, pool.cuh).  Same bits as the dense schedule.
 #include <cstdio>
 #include <cstring>
 
 #include "common.cuh"
 #include "pool.cuh"
+#include "tc.cuh"
 
 namespace ssd3d {
 
@@ -44,7 +43,7 @@ constexpr int TC_EPI_WARP0 = TC_PROD_WARP0 + TC_PROD_WARPS;   // warps 6..13: ep
 constexpr int TC_EPI_WARPS = 8;
 constexpr int TC_THREADS = (TC_EPI_WARP0 + TC_EPI_WARPS) * 32;
 constexpr int TC_MAX_STAGES = 4;
-constexpr int TC_MAX_AKB = 4;            // A-stationary mode: k-blocks of an m-tile resident at once (K <= 256)
+constexpr int TC_MAX_AKB = 4;            // A-stationary mode: k-blocks of the resident A tile (K <= 256)
 constexpr uint32_t TC_A_BYTES = TC_BM * TC_BK * 2;   // one A tile (hi or lo): 16 KiB
 
 struct TcParams {
@@ -67,9 +66,9 @@ struct TcParams {
     // g_points = z (row pitch g_ldz, this scale's columns), g_c = first-layer width (= K of this layer), g_wx = Wx*s [3][g_c]
     // astat ("A-stationary", gather modes): the produced A tile of an m-tile (all its k-blocks) stays in shared memory
     // while the CTA sweeps that m-tile's n-tiles, so the producers build it once instead of once per n-tile; only the
-    // weights travel through the ring.  Tiles are then enumerated m-major per CTA.
-    int astat;       // 0: A through the ring; 1: one resident A tile; 2: TWO resident A tiles (the producers build m-tile
-                     // i+1 while the MMAs of m-tile i run -- with one buffer the two strictly alternate)
+    // weights travel through the ring.  Tiles are then enumerated m-major per CTA.  (A second resident tile, built under
+    // the MMAs of the first, was measured slower and removed: DESIGN.md section 8.)
+    int astat;       // 0: A through the ring; 1: one resident A tile
     int gather, g_n, g_c, g_m, g_ns, g_ldz;
     const float *g_xyz, *g_points, *g_new_xyz, *g_wx;
     const int *g_idx;
@@ -81,128 +80,6 @@ struct TcParams {
     const int *units;
     int unit_pool;
 };
-
-// ---- PTX wrappers ---------------------------------------------------------------------------------------
-__device__ __forceinline__ void tma_load_2d(uint32_t dst, const CUtensorMap *map, int x, int y, uint32_t bar)
-{
-    asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-                 ::"r"(dst), "l"(map), "r"(bar), "r"(x), "r"(y) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint32_t bar)
-{
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void umma_bf16(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t acc)
-{
-    asm volatile(
-        "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-        ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(acc) : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint32_t bar)
-{
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&r)[32])
-{
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-        "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-        "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]),
-          "=r"(r[8]), "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]),
-          "=r"(r[16]), "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]),
-          "=r"(r[24]), "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-        : "r"(taddr));
-    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tma_store_2d(const CUtensorMap *map, uint32_t src, int x, int y)
-{
-    asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];"
-                 ::"l"(map), "r"(src), "r"(x), "r"(y) : "memory");
-}
-__device__ __forceinline__ void tma_store_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-__device__ __forceinline__ void tma_store_wait_read() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
-__device__ __forceinline__ void tma_store_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
-__device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-// K-major, 128B-swizzled operand tile: rows are 128 bytes, 8-row groups are 1024 bytes apart (SBO), version 1
-__device__ __forceinline__ uint64_t umma_desc(uint32_t smem_addr)
-{
-    return (uint64_t)((smem_addr & 0x3FFFFu) >> 4) | (1ull << 16) | ((uint64_t)(1024 >> 4) << 32) | (1ull << 46) |
-           (2ull << 61);
-}
-
-// ---- epilogue helpers ---------------------------------------------------------------------------------------
-// order-preserving float <-> uint map (so that an unsigned redux.max is a float max, also for negative values)
-__device__ __forceinline__ uint32_t f2ord(float x)
-{
-    const uint32_t b = __float_as_uint(x);
-    return (b & 0x80000000u) ? ~b : (b | 0x80000000u);
-}
-__device__ __forceinline__ float ord2f(uint32_t u)
-{
-    return __uint_as_float((u & 0x80000000u) ? (u & 0x7fffffffu) : ~u);
-}
-__device__ __forceinline__ void split_pair(float x0, float x1, uint32_t &hw, uint32_t &lw)
-{
-    asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(hw) : "f"(x1), "f"(x0));       // {x1 : x0} like two adjacent bf16
-    const float h0 = __uint_as_float(hw << 16), h1 = __uint_as_float(hw & 0xffff0000u);
-    asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(lw) : "f"(x1 - h1), "f"(x0 - h0));
-}
-
-// Max-pool of one 32-column chunk over runs of POOL rows (tf.reduce_max(axis=2), layers_util.py:178) + mask (:180).
-// A thread holds one row; the rows of a group are lanes of a warp (POOL <= 32) or of 2-4 warps (64, 128).
-template <int POOL>
-__device__ __forceinline__ void pooled_chunk(const TcParams &p, float (&v)[32], int lane, int q, int h, int mt,
-                                             int col0, float *xs /* [2 halves][4 quarters][32] */)
-{
-    constexpr int GP = POOL >= 32 ? 32 : POOL;       // lanes per group inside a warp
-    constexpr int KEEP = 32 / GP;                    // columns a lane ends up owning
-    warp_colmax_transpose<GP>(v, lane);              // lane owns columns (lane % GP) * KEEP + k in v[k]
-    if (POOL > 32) {                                 // combine the 2 (4) warps that share a group
-        constexpr int WPG = POOL > 32 ? POOL / 32 : 1;
-        xs[(h * 4 + q) * 32 + lane] = v[0];
-        asm volatile("bar.sync %0, 128;" ::"r"(2 + h) : "memory");      // the 4 quarter-warps of this column half
-        if ((q % WPG) == 0) {
-#pragma unroll
-            for (int w = 1; w < WPG; w++) v[0] = fmaxf(v[0], xs[(h * 4 + q + w) * 32 + lane]);
-        }
-        asm volatile("bar.sync %0, 128;" ::"r"(2 + h) : "memory");      // xs reusable by the next chunk
-        if ((q % WPG) != 0) return;
-    }
-    const long gg = (long)mt * (TC_BM / POOL) + (q * 32 + lane) / POOL;
-    if (gg * POOL >= p.rows) return;
-    const bool masked = p.rowmask && p.rowmask[gg] == 0;
-#pragma unroll
-    for (int k = 0; k < KEEP; k++) {
-        const int col = col0 + (lane % GP) * KEEP + k;
-        if (col >= p.n) continue;
-        const float mx = masked ? 0.0f : v[k];
-        if (p.out_f32) p.out_f32[(size_t)gg * p.ld_f32 + col] = mx;
-        if (p.out_hi) {
-            const __nv_bfloat16 hb = __float2bfloat16_rn(mx);
-            p.out_hi[(size_t)gg * p.ld_split + col] = hb;
-            p.out_lo[(size_t)gg * p.ld_split + col] = __float2bfloat16_rn(mx - __bfloat162float(hb));
-        }
-    }
-}
-
-// Unit-list twin of pooled_chunk<8>: lanes 8u' .. 8u'+7 of a warp hold one unit; its column maxima go to the unit's GROUP row.
-__device__ __forceinline__ void pooled_units_chunk(const TcParams &p, float (&v)[32], int lane, int q, int mt, int col0, int nunits)
-{
-    warp_colmax_transpose<8>(v, lane);               // lane owns columns (lane % 8) * 4 + k of its unit in v[k]
-    const int ui = mt * (TC_BM / 8) + ((q * 32 + lane) >> 3);
-    if (ui >= nunits) return;
-    const int group = __ldg(p.units + 1 + ui) >> 4;
-#pragma unroll
-    for (int k = 0; k < 4; k++) {
-        const int col = col0 + (lane & 7) * 4 + k;
-        if (col >= p.n) continue;
-        atomicMax(reinterpret_cast<unsigned int *>(p.out_f32 + (size_t)group * p.ld_f32 + col), __float_as_uint(v[k]) & 0x7fffffffu);
-    }
-}
 
 // Developer instrumentation (nvcc -DTC_PROFILE): CTA 0 accumulates, per role, the cycles spent waiting on each barrier
 // and the cycles spent working; printed by the launcher.  Slots: 0 total | 1 tma wait-empty | 2 mma wait-afull |
@@ -228,7 +105,7 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap map_ahi, const __grid_const
     const uint32_t b_bytes = (uint32_t)p.bn * TC_BK * 2;
     const int nkb = (p.kp + TC_BK - 1) / TC_BK;
     const uint32_t a_tile = (uint32_t)nkb * 2u * TC_A_BYTES;                        // one resident A tile: [nkb] x { A_hi | A_lo }
-    const uint32_t a_region = (uint32_t)p.astat * a_tile;
+    const uint32_t a_region = p.astat ? a_tile : 0u;
     const uint32_t stage_bytes = (p.astat ? 0u : 2 * TC_A_BYTES) + 2 * b_bytes;     // ring stage
     const uint32_t b_off = p.astat ? 0u : 2 * TC_A_BYTES;                           // B_hi inside a stage
     // 1 KiB alignment by pointer arithmetic on the __shared__ array (an integer round-trip would demote every access
@@ -242,7 +119,7 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap map_ahi, const __grid_const
     float *s_wx = s_shift + ncov;                                        // [3][kp] (hoisted mode only)
 
     __shared__ unsigned long long full_bar[TC_MAX_STAGES], empty_bar[TC_MAX_STAGES], tfull_bar[2], tempty_bar[2];
-    __shared__ unsigned long long afull_bar[2 * TC_MAX_AKB], aempty_bar[2 * TC_MAX_AKB];   // [A buffer][k-block]
+    __shared__ unsigned long long afull_bar[TC_MAX_AKB], aempty_bar[TC_MAX_AKB];   // per k-block of the resident A tile
     __shared__ uint32_t tmem_base_smem;
     __shared__ float pool_xs[2 * 4 * 32];
 
@@ -267,14 +144,11 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap map_ahi, const __grid_const
     if (threadIdx.x == 0) {
         // full barrier: the TMA thread's expect_tx arrival (+ one arrival per producer warp in gather mode)
         for (int s = 0; s < p.stages; s++) { mbar_init(smem_u32(&full_bar[s]), (p.gather && !p.astat) ? 1 + TC_PROD_WARPS : 1); mbar_init(smem_u32(&empty_bar[s]), 1); }
-        for (int k = 0; k < 2 * TC_MAX_AKB; k++) { mbar_init(smem_u32(&afull_bar[k]), TC_PROD_WARPS); mbar_init(smem_u32(&aempty_bar[k]), 1); }
+        for (int k = 0; k < TC_MAX_AKB; k++) { mbar_init(smem_u32(&afull_bar[k]), TC_PROD_WARPS); mbar_init(smem_u32(&aempty_bar[k]), 1); }
         for (int a = 0; a < 2; a++) { mbar_init(smem_u32(&tfull_bar[a]), 1); mbar_init(smem_u32(&tempty_bar[a]), TC_EPI_WARPS); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        fence_mbar_init_cluster();
     }
-    if (warp == 2) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_smem)), "r"(512u) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
+    if (warp == 2) tmem_alloc(&tmem_base_smem, 512u);
     for (int i = threadIdx.x; i < ncov; i += TC_THREADS) {      // columns >= n: scale = shift = 0 -> exact zeros
         s_scale[i] = i < p.n ? __ldg(p.scale + i) : 0.0f;
         s_shift[i] = i < p.n ? __ldg(p.shift + i) : 0.0f;
@@ -321,8 +195,7 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap map_ahi, const __grid_const
         // ===== MMA issuer: the whole warp runs the loop (uniform control flow keeps descriptors in uniform registers
         // and tcgen05.mma free of a per-instruction election loop), one elected lane issues =====
         {
-            // instruction descriptor: D=f32, A=B=bf16, both K-major, N = bn, M = 128
-            const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(p.bn >> 3) << 17) | ((uint32_t)(TC_BM >> 4) << 24);
+            const uint32_t idesc = umma_idesc_bf16(p.bn);
             int it = 0, tcount = 0, mi = 0, mt, nt;
             TCP_DECL;
             for (int i = 0; tile_at(i, mt, nt); i++, tcount++) {
@@ -336,27 +209,21 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap map_ahi, const __grid_const
                 for (int kb = 0; kb < nkb; kb++, it++) {
                     const int s = it % p.stages;
                     TCP(5);
-                    const int ab = p.astat == 2 ? (mi & 1) : 0;                 // resident A buffer of this m-tile
-                    const uint32_t aph = (uint32_t)(p.astat == 2 ? (mi >> 1) : mi) & 1u;   // how often it has been used before
-                    if (p.astat && nt == 0) mbar_wait_cta(smem_u32(&afull_bar[ab * TC_MAX_AKB + kb]), aph);   // this m-tile's A k-block
+                    if (p.astat && nt == 0) mbar_wait_cta(smem_u32(&afull_bar[kb]), (uint32_t)mi & 1u);   // this m-tile's A k-block
                     TCP(2);
                     mbar_wait_cta(smem_u32(&full_bar[s]), (uint32_t)(it / p.stages) & 1u);
                     TCP(3);
                     tc_fence_after();
                     const uint32_t base = smem_u32(ring + (size_t)s * stage_bytes);
-                    const uint32_t abase = p.astat ? smem_u32(smem) + (uint32_t)ab * a_tile + (uint32_t)kb * 2u * TC_A_BYTES : base;
+                    const uint32_t abase = p.astat ? smem_u32(smem) + (uint32_t)kb * 2u * TC_A_BYTES : base;
                     const int ksteps = min(TC_BK, p.kp - kb * TC_BK) / 16;
-                    const uint64_t a_hi = umma_desc(abase), a_lo = umma_desc(abase + TC_A_BYTES);
-                    const uint64_t b_hi = umma_desc(base + b_off), b_lo = umma_desc(base + b_off + b_bytes);
+                    const uint64_t a_hi = umma_desc(abase, 128), a_lo = umma_desc(abase + TC_A_BYTES, 128);
+                    const uint64_t b_hi = umma_desc(base + b_off, 128), b_lo = umma_desc(base + b_off + b_bytes, 128);
                     if (elect_one()) {
-                        for (int ks = 0; ks < ksteps; ks++) {          // +2 per k-step: 32 bytes in the address field
-                            const uint32_t first = (kb | ks) ? 1u : 0u;
-                            umma_bf16(d_tmem, a_hi + 2 * ks, b_hi + 2 * ks, idesc, first);
-                            umma_bf16(d_tmem, a_lo + 2 * ks, b_hi + 2 * ks, idesc, 1u);
-                            umma_bf16(d_tmem, a_hi + 2 * ks, b_lo + 2 * ks, idesc, 1u);
-                        }
+                        for (int ks = 0; ks < ksteps; ks++)           // +2 per k-step: 32 bytes in the address field
+                            umma_bf16x3(d_tmem, a_hi + 2 * ks, a_lo + 2 * ks, b_hi + 2 * ks, b_lo + 2 * ks, idesc, (kb | ks) ? 1u : 0u);
                         umma_commit(smem_u32(&empty_bar[s]));   // ring stage free once these MMAs retire
-                        if (p.astat && last_nt) umma_commit(smem_u32(&aempty_bar[ab * TC_MAX_AKB + kb]));   // A k-block free again
+                        if (p.astat && last_nt) umma_commit(smem_u32(&aempty_bar[kb]));   // A k-block free again
                     }
                     __syncwarp();
                 }
@@ -425,39 +292,22 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap map_ahi, const __grid_const
                     }
                     // (loads already in flight) wait for the slot: ring stage, or this k-block of the resident A tile
                     if (warp == TC_PROD_WARP0) TCP(7);
-                    const int ab = p.astat == 2 ? (mi & 1) : 0;
-                    const uint32_t aph = (uint32_t)(p.astat == 2 ? (mi >> 1) : mi) & 1u;
-                    if (p.astat) mbar_wait_cta(smem_u32(&aempty_bar[ab * TC_MAX_AKB + kb]), aph ^ 1u);
+                    if (p.astat) mbar_wait_cta(smem_u32(&aempty_bar[kb]), ((uint32_t)mi & 1u) ^ 1u);
                     else mbar_wait_cta(smem_u32(&empty_bar[s]), ((uint32_t)(it / p.stages) & 1u) ^ 1u);
                     if (warp == TC_PROD_WARP0) TCP(6);
-                    uint8_t *rowp = (p.astat ? smem + (size_t)ab * a_tile + (size_t)kb * 2 * TC_A_BYTES : ring + (size_t)s * stage_bytes) + row_off;
+                    uint8_t *rowp = (p.astat ? smem + (size_t)kb * 2 * TC_A_BYTES : ring + (size_t)s * stage_bytes) + row_off;
 #pragma unroll
                     for (int cc = 0; cc < 4; cc++) {
                         const int c16 = c16_0 + cc;
                         const int k0 = kb * TC_BK + c16 * 8;
                         if (k0 >= p.kp) break;
-                        if (hoisted) {                                   // relu(z + d . Wx'); rows beyond the tensor stay 0
-#pragma unroll
-                            for (int e4 = 0; e4 < 8; e4 += 4) {
-                                const float4 w0 = *reinterpret_cast<const float4 *>(s_wx + k0 + e4);
-                                const float4 w1 = *reinterpret_cast<const float4 *>(s_wx + p.kp + k0 + e4);
-                                const float4 w2 = *reinterpret_cast<const float4 *>(s_wx + 2 * p.kp + k0 + e4);
-                                f[cc][e4 + 0] = fmaxf(fmaf(dz, w2.x, fmaf(dy, w1.x, fmaf(dx, w0.x, f[cc][e4 + 0]))), 0.0f);
-                                f[cc][e4 + 1] = fmaxf(fmaf(dz, w2.y, fmaf(dy, w1.y, fmaf(dx, w0.y, f[cc][e4 + 1]))), 0.0f);
-                                f[cc][e4 + 2] = fmaxf(fmaf(dz, w2.z, fmaf(dy, w1.z, fmaf(dx, w0.z, f[cc][e4 + 2]))), 0.0f);
-                                f[cc][e4 + 3] = fmaxf(fmaf(dz, w2.w, fmaf(dy, w1.w, fmaf(dx, w0.w, f[cc][e4 + 3]))), 0.0f);
-                            }
-                        }
-                        uint32_t hw[4], lw[4];
-#pragma unroll
-                        for (int t = 0; t < 4; t++) split_pair(f[cc][2 * t], f[cc][2 * t + 1], hw[t], lw[t]);
+                        if (hoisted) hoist_relu8(f[cc], dx, dy, dz, s_wx + k0, p.kp);   // rows beyond the tensor stay 0
                         const uint32_t off = (uint32_t)((c16 ^ (r & 7)) << 4);
-                        *reinterpret_cast<uint4 *>(rowp + off) = make_uint4(hw[0], hw[1], hw[2], hw[3]);
-                        *reinterpret_cast<uint4 *>(rowp + TC_A_BYTES + off) = make_uint4(lw[0], lw[1], lw[2], lw[3]);
+                        split8_store(f[cc], rowp + off, rowp + TC_A_BYTES + off);
                     }
                     fence_async_smem();                                   // generic-proxy stores -> visible to the tensor core
                     __syncwarp();
-                    if (lane == 0) mbar_arrive(smem_u32(p.astat ? &afull_bar[ab * TC_MAX_AKB + kb] : &full_bar[s]));
+                    if (lane == 0) mbar_arrive(smem_u32(p.astat ? &afull_bar[kb] : &full_bar[s]));
                 }
                 mi++;
             }
@@ -515,12 +365,8 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap map_ahi, const __grid_const
                     } else {                                           // two 64-byte-row blocks (hi, lo), SWIZZLE_64B
 #pragma unroll
                         for (int c = 0; c < 4; c++) {
-                            uint32_t hw[4], lw[4];
-#pragma unroll
-                            for (int t = 0; t < 4; t++) split_pair(v[8 * c + 2 * t], v[8 * c + 2 * t + 1], hw[t], lw[t]);
                             const uint32_t off = (uint32_t)lane * 64u + (uint32_t)((c ^ ((lane >> 1) & 3)) << 4);
-                            *reinterpret_cast<uint4 *>(blk + off) = make_uint4(hw[0], hw[1], hw[2], hw[3]);
-                            *reinterpret_cast<uint4 *>(blk + 2048 + off) = make_uint4(lw[0], lw[1], lw[2], lw[3]);
+                            split8_store(v + 8 * c, blk + off, blk + 2048 + off);
                         }
                         fence_async_smem();
                         __syncwarp();
@@ -551,24 +397,16 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap map_ahi, const __grid_const
 #pragma unroll
                             for (int j8 = 0; j8 < 32; j8 += 8) {
                                 if (col0 + j8 >= p.ld_split) break;
-                                uint32_t hw[4], lw[4];
-#pragma unroll
-                                for (int t = 0; t < 4; t++) split_pair(v[j8 + 2 * t], v[j8 + 2 * t + 1], hw[t], lw[t]);
-                                *reinterpret_cast<uint4 *>(dh + j8) = make_uint4(hw[0], hw[1], hw[2], hw[3]);
-                                *reinterpret_cast<uint4 *>(dl + j8) = make_uint4(lw[0], lw[1], lw[2], lw[3]);
+                                split8_store(v + j8, dh + j8, dl + j8);
                             }
                         }
                     }
-                } else if (p.unit_pool) {
-                    pooled_units_chunk(p, v, lane, q, mt, col0, nunits);
-                } else {
-                    switch (p.pool) {
-                        case 8: pooled_chunk<8>(p, v, lane, q, h, mt, col0, pool_xs); break;
-                        case 16: pooled_chunk<16>(p, v, lane, q, h, mt, col0, pool_xs); break;
-                        case 32: pooled_chunk<32>(p, v, lane, q, h, mt, col0, pool_xs); break;
-                        case 64: pooled_chunk<64>(p, v, lane, q, h, mt, col0, pool_xs); break;
-                        default: pooled_chunk<128>(p, v, lane, q, h, mt, col0, pool_xs); break;
-                    }
+                } else if (p.unit_pool) {                              // lanes 8u' .. 8u'+7 of a warp hold one unit
+                    const int ui = mt * (TC_BM / 8) + ((q * 32 + lane) >> 3);
+                    const bool ok = ui < nunits;
+                    pool_units<false>(p, v, lane, col0, p.n, nullptr, nullptr, ok ? __ldg(p.units + 1 + ui) >> 4 : 0, ok);
+                } else {                                               // the 4 quarter-warps of column half h: barrier 2 + h
+                    pool_rows<false>(p.pool, p, p.rowmask, v, lane, q, mt, col0, p.n, nullptr, nullptr, pool_xs + h * 4 * 32, 2 + h);
                 }
             }
             tc_fence_before();
@@ -582,7 +420,7 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap map_ahi, const __grid_const
     __syncthreads();
     if (warp == 2) {
         tc_fence_after();
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
+        tmem_dealloc(tmem_base, 512u);
     }
 }
 
@@ -717,7 +555,8 @@ group_concat_split_kernel(long rows, int n, int c, int m, int ns, const float *_
 // For wide layers (K >= 256, 3DSSD layer 4) the A-stationary in-kernel producers starve the tensor pipe -- 128 KiB of
 // resident operand leave room for two narrow weight stages -- while this elementwise pass runs at memory speed on the whole
 // machine and the GEMM then takes the plain TMA-fed path.  One warp per row, one 8-column chunk per lane per step.
-__global__ void __launch_bounds__(256)
+// 8 blocks per SM: a full SM of warps for this memory-bound pass (the compiler would otherwise take 43 registers).
+__global__ void __launch_bounds__(256, 8)
 hoist_expand_split_kernel(long rows, int n, int n1, int m, int ns, const float *__restrict__ xyz, const float *__restrict__ z,
                           int ldz, const float *__restrict__ wx, const float *__restrict__ new_xyz,
                           const int *__restrict__ idx, const int *__restrict__ units, __nv_bfloat16 *__restrict__ hi,
@@ -755,16 +594,8 @@ hoist_expand_split_kernel(long rows, int n, int n1, int m, int ns, const float *
 #pragma unroll
                 for (int e = 0; e < 8; e++) f[e] = k0 + e < n1 ? __ldg(zr + k0 + e) : 0.0f;
             }
-            uint32_t hw[4], lw[4];
-#pragma unroll
-            for (int e = 0; e < 8; e++) {
-                const float v = fmaf(dz, hx_wx[2 * kp + k0 + e], fmaf(dy, hx_wx[kp + k0 + e], fmaf(dx, hx_wx[k0 + e], f[e])));
-                f[e] = k0 + e < n1 ? fmaxf(v, 0.0f) : 0.0f;
-            }
-#pragma unroll
-            for (int t = 0; t < 4; t++) split_pair(f[2 * t], f[2 * t + 1], hw[t], lw[t]);
-            *reinterpret_cast<uint4 *>(hi + (size_t)row * kp + k0) = make_uint4(hw[0], hw[1], hw[2], hw[3]);
-            *reinterpret_cast<uint4 *>(lo + (size_t)row * kp + k0) = make_uint4(lw[0], lw[1], lw[2], lw[3]);
+            hoist_relu8(f, dx, dy, dz, hx_wx + k0, kp);
+            split8_store(f, hi + (size_t)row * kp + k0, lo + (size_t)row * kp + k0);
         }
     }
 }
@@ -880,30 +711,13 @@ static int linear_tc_launch(long rows, int kp, int n, const void *a_hi, const vo
                (g && g->wx ? (size_t)3 * kp * sizeof(float) : 0);
     };
     // gather modes keep the produced A tile resident (A-stationary) when all its k-blocks fit next to a >= 2-stage
-    // weight ring: the producers then build it once per m-tile, not once per (m, n) tile
+    // weight ring: the producers then build it once per m-tile, not once per (m, n) tile.  A second resident tile (the
+    // producers building m-tile i+1 under the MMAs of m-tile i) had to be paid for with the TMA store blocks and lost on
+    // the layer-3 shapes; it was removed (DESIGN.md section 8 keeps the measurement).
     int bn = 0, stages = 0;
     p.astat = 0;
     if (g && nkb <= TC_MAX_AKB) {
         const size_t a_tile = (size_t)nkb * 2 * TC_A_BYTES;
-        // TWO resident A tiles would let the producers build m-tile i+1 while the MMAs of m-tile i run (with one tile the two
-        // alternate).  The second tile has to be paid for with the per-warp TMA store blocks -- split outputs then leave as
-        // direct 16-byte stores -- and that trade LOSES on the layer-3 shapes: 33 / 43 / 47 us with one tile + TMA stores vs
-        // 57 / 71 / 80 us with two tiles + direct stores (round 2, profiles/r02_bench_1gpu_run4_two_a_tiles.json).  The kernel
-        // keeps the capability (TcParams::astat == 2); the planner does not choose it.
-        constexpr bool kTwoATiles = false;
-        if (kTwoATiles && pool <= 1 && want_split && !want_f32) {
-            const bool saved = tma_store;
-            tma_store = false;
-            const int b = ncover < 128 ? ncover : 128;
-            const size_t need = 2 * a_tile + misc_bytes(b);
-            if (need + 2 * (size_t)(2 * b * TC_BK * 2) <= budget) {
-                bn = b;
-                stages = (int)((budget - need) / (size_t)(2 * b * TC_BK * 2));
-                p.astat = 2;
-            } else {
-                tma_store = saved;
-            }
-        }
         const int cands[4] = {256, 128, 96, 64};            // widest tile first: a tcgen05.mma has a fixed cost per instruction
         for (int ci = tma_store ? 1 : 0; ci < 4 && !bn; ci++) {
             const int cand = cands[ci];
@@ -916,7 +730,6 @@ static int linear_tc_launch(long rows, int kp, int n, const void *a_hi, const vo
             }
         }
     }
-    p.tma_store = tma_store ? 1 : 0;
     if (!bn) {
         const int bn_cap = tma_store ? 128 : 256;
         bn = ncover < bn_cap ? ncover : bn_cap;
@@ -926,7 +739,7 @@ static int linear_tc_launch(long rows, int kp, int n, const void *a_hi, const vo
     p.n_tiles = (ncover + p.bn - 1) / p.bn;
     p.m_tiles = (int)((rows + TC_BM - 1) / TC_BM);
     const size_t stage_bytes = (p.astat ? 0 : 2 * (size_t)TC_A_BYTES) + 2 * (size_t)p.bn * TC_BK * 2;
-    const size_t pool_bytes = misc_bytes(p.bn) + (size_t)p.astat * nkb * 2 * TC_A_BYTES;
+    const size_t pool_bytes = misc_bytes(p.bn) + (p.astat ? (size_t)nkb * 2 * TC_A_BYTES : 0);
     SSD3D_REQUIRE((size_t)p.n_tiles * p.bn <= 4096, "linear_tc: n=%d too wide for the staged scale/shift", n);
     if (stages > TC_MAX_STAGES) stages = TC_MAX_STAGES;
     SSD3D_REQUIRE(stages >= 2, "linear_tc: tile does not fit shared memory");

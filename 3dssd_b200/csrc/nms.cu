@@ -17,12 +17,6 @@ namespace ssd3d {
 constexpr int NMS_THREADS = 256;
 constexpr int NMS_MAX_N = 512;
 
-__device__ __forceinline__ uint32_t nms_f2ord(float x)
-{
-    const uint32_t b = __float_as_uint(x);
-    return (b & 0x80000000u) ? ~b : (b | 0x80000000u);
-}
-
 __global__ void __launch_bounds__(NMS_THREADS)
 bev_nms_kernel(int n, int npow2, const float *__restrict__ boxes, const float *__restrict__ scores, float iou_thr,
                int max_out, int cls_id, float *__restrict__ out_block, int *__restrict__ out_cnt)
@@ -39,7 +33,7 @@ bev_nms_kernel(int n, int npow2, const float *__restrict__ boxes, const float *_
 
     // ---- sort keys: (score desc, index asc)  ==  descending on (ord(score) << 32 | ~index)
     for (int i = tid; i < npow2; i += NMS_THREADS)
-        keys[i] = i < n ? (((unsigned long long)nms_f2ord(sc[i]) << 32) | (unsigned long long)(0xffffffffu - (uint32_t)i)) : 0ull;
+        keys[i] = i < n ? (((unsigned long long)f2ord(sc[i]) << 32) | (unsigned long long)(0xffffffffu - (uint32_t)i)) : 0ull;
     __syncthreads();
     for (int k = 2; k <= npow2; k <<= 1)
         for (int j = k >> 1; j > 0; j >>= 1) {

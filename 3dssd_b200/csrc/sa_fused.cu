@@ -25,13 +25,13 @@
 // zero-fills (= the cnt == 0 mask of layers_util.py:180).  Same bits as the dense schedule, 4-8x fewer rows on KITTI-like
 // clouds (DESIGN.md section 3.4).
 //
-// Precision: same bf16 hi/lo split and 3-MMA scheme as mlp_tc.cu.
-#include <cuda_bf16.h>
+// Precision: the bf16 hi/lo split and 3-MMA scheme of tc.cuh, as in mlp_tc.cu.
 #include <cstdio>
 #include <cstring>
 
 #include "common.cuh"
 #include "pool.cuh"
+#include "tc.cuh"
 
 namespace ssd3d {
 
@@ -74,48 +74,6 @@ struct SfParams {
     int pool_first;                  // caller guarantees scale >= 0 in the LAST layer: pool raw accumulators, affine after
 };
 
-__device__ __forceinline__ void sf_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void sf_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void sf_fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-// K-major operand descriptor; rb = bytes per row = swizzle span (128 -> SWIZZLE_128B, 64 -> _64B, 32 -> _32B),
-// 8-row groups are 8*rb bytes apart (SBO), descriptor version 1
-__device__ __forceinline__ uint64_t sf_desc(uint32_t smem_addr, int rb)
-{
-    const uint64_t layout = rb == 128 ? 2ull : (rb == 64 ? 4ull : 6ull);
-    return (uint64_t)((smem_addr & 0x3FFFFu) >> 4) | (1ull << 16) | ((uint64_t)((8 * rb) >> 4) << 32) | (1ull << 46) |
-           (layout << 61);
-}
-__device__ __forceinline__ void sf_mma(uint32_t d_tmem, uint64_t a, uint64_t b, uint32_t idesc, uint32_t acc)
-{
-    asm volatile(
-        "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-        ::"r"(d_tmem), "l"(a), "l"(b), "r"(idesc), "r"(acc) : "memory");
-}
-__device__ __forceinline__ void sf_commit(uint32_t bar)
-{
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void sf_tmem_ld32(uint32_t taddr, uint32_t (&r)[32])
-{
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-        "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-        "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]),
-          "=r"(r[8]), "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]),
-          "=r"(r[16]), "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]),
-          "=r"(r[24]), "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-        : "r"(taddr));
-    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
-// x = hi + lo with hi = bf16(x), lo = bf16(x - hi); two values per call, packed {x1 : x0} like two adjacent bf16
-__device__ __forceinline__ void sf_split_pair(float x0, float x1, uint32_t &hw, uint32_t &lw)
-{
-    asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(hw) : "f"(x1), "f"(x0));
-    const float h0 = __uint_as_float(hw << 16), h1 = __uint_as_float(hw & 0xffff0000u);
-    asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(lw) : "f"(x1 - h1), "f"(x0 - h0));
-}
 // Where row r of a 128-row operand tile lives.  An A buffer is laid out as k-blocks of { hi tile | lo tile }
 // (128 rows x rb bytes each), each tile in the canonical K-major swizzled layout of span rb: 16-byte chunk j of
 // row r sits at chunk j ^ ((r >> log2(128/rb)) & (rb/16 - 1)).  The first nfull blocks are 64 wide (rb = 128),
@@ -147,13 +105,6 @@ struct SfRowMap {
         return base_t + row_t + (((uint32_t)(c16g - full8) ^ xor_t) << 4);
     }
 };
-__device__ __forceinline__ void sf_bar_sync(int id, int nthreads) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory"); }
-__device__ __forceinline__ uint32_t sf_f2ord(float x)
-{
-    const uint32_t b = __float_as_uint(x);
-    return (b & 0x80000000u) ? ~b : (b | 0x80000000u);
-}
-__device__ __forceinline__ float sf_ord2f(uint32_t u) { return __uint_as_float((u & 0x80000000u) ? (u & 0x7fffffffu) : ~u); }
 
 // ---- shape policies -------------------------------------------------------------------------------------------------
 // The kernel body is written once against a policy C that answers every shape question (layer count, padded K / N of a
@@ -163,6 +114,9 @@ __device__ __forceinline__ float sf_ord2f(uint32_t u) { return __uint_as_float((
 // literal: profiling the dynamic kernel showed ~50% of its issued instructions to be integer / branch / uniform-register
 // bookkeeping of exactly these questions (profiles/r02_fused_instruction_mix.txt).
 __host__ __device__ constexpr int sf_r16(int x) { return (x + 15) / 16 * 16; }
+// Operand layout of a layer with padded K = kp: kp / 64 full 64-wide k-blocks of 128-byte rows + a tail block whose rows
+// are sf_rbt_of(kp) = 32 / 64 / 128 bytes for a remainder of 16 / 32 / 48 columns (must match params._k_blocks).
+// An operand buffer holds { hi | lo } tiles of 128 rows per block, 1 KiB granular.
 __host__ __device__ constexpr int sf_rbt_of(int kp) { return kp % 64 == 0 ? 0 : (kp % 64 <= 16 ? 32 : (kp % 64 <= 32 ? 64 : 128)); }
 __host__ __device__ constexpr uint32_t sf_abuf_of(int kp)
 {
@@ -228,68 +182,6 @@ __device__ long long sf_prof[16];
 #define SF_T(i) do { } while (0)
 #endif
 
-// Max-pool of one 32-column chunk over runs of POOL rows + mask + store.  AFTER: v holds RAW accumulators and the folded
-// affine + ReLU is applied to the pooled values only (valid when the layer's scale is >= 0: fma(x, s, t) is then monotone
-// non-decreasing in x, so max_i relu(fma(x_i, s, t)) == relu(fma(max_i x_i, s, t)) exactly) -- 1/POOL of the epilogue math.
-template <int POOL, bool AFTER>
-__device__ __forceinline__ void sf_pool_store(const SfParams &p, float (&v)[32], int lane, int q, int tile,
-                                              int col0, int nout, float *xs, int wg_bar, const float *sc, const float *sh)
-{
-    constexpr int GP = POOL >= 32 ? 32 : POOL;
-    constexpr int KEEP = 32 / GP;
-    constexpr int WPG = POOL > 32 ? POOL / 32 : 1;
-    warp_colmax_transpose<GP>(v, lane);                   // lane owns columns (lane % GP) * KEEP + k in v[k]
-    if (POOL > 32) {                                      // groups spanning 2 or 4 warps: combine through shared memory
-        xs[q * 32 + lane] = v[0];
-        sf_bar_sync(wg_bar, 128);
-        if ((q % WPG) == 0) {
-#pragma unroll
-            for (int w = 1; w < WPG; w++) v[0] = fmaxf(v[0], xs[(q + w) * 32 + lane]);
-        }
-        sf_bar_sync(wg_bar, 128);
-        if ((q % WPG) != 0) return;
-    }
-    const int gg = tile * (128 / POOL) + (q * 32 + lane) / POOL;
-    if ((long)gg * POOL >= p.rows) return;
-    const bool masked = p.cnt && p.cnt[gg] == 0;
-#pragma unroll
-    for (int k = 0; k < KEEP; k++) {
-        const int cc = (lane % GP) * KEEP + k;
-        const int col = col0 + cc;
-        if (col >= nout) continue;
-        float mx = v[k];
-        if (AFTER) mx = fmaxf(fmaf(mx, sc[col0 + cc], sh[col0 + cc]), 0.0f);
-        mx = masked ? 0.0f : mx;
-        if (p.out_f32) asm volatile("st.global.f32 [%0], %1;" ::"l"(p.out_f32 + (size_t)gg * p.ld_f32 + col), "f"(mx) : "memory");
-        if (p.out_hi) {
-            const __nv_bfloat16 hb = __float2bfloat16_rn(mx);
-            const __nv_bfloat16 lb = __float2bfloat16_rn(mx - __bfloat162float(hb));
-            asm volatile("st.global.b16 [%0], %1;" ::"l"(p.out_hi + (size_t)gg * p.ld_split + col), "h"(__bfloat16_as_ushort(hb)) : "memory");
-            asm volatile("st.global.b16 [%0], %1;" ::"l"(p.out_lo + (size_t)gg * p.ld_split + col), "h"(__bfloat16_as_ushort(lb)) : "memory");
-        }
-    }
-}
-
-// Unit-list mode: a unit is 8 rows = 8 consecutive lanes.  Max over the unit, then atomicMax into out[group]: post-ReLU
-// values are >= 0, where the unsigned order of the bit patterns is the float order (a -0.0 is folded to +0.0), and the
-// caller zero-fills the output, which is also the result of a group without hits (the mask of layers_util.py:180).
-template <bool AFTER>
-__device__ __forceinline__ void sf_pool_atomic8(const SfParams &p, float (&v)[32], int lane, int col0, int nout, const float *sc,
-                                                const float *sh, int group, bool ok)
-{
-    warp_colmax_transpose<8>(v, lane);                    // lane owns columns (lane % 8) * 4 + k of its unit in v[k]
-    if (!ok) return;
-#pragma unroll
-    for (int k = 0; k < 4; k++) {
-        const int cc = (lane & 7) * 4 + k;
-        const int col = col0 + cc;
-        if (col >= nout) continue;
-        float mx = v[k];
-        if (AFTER) mx = fmaxf(fmaf(mx, sc[col0 + cc], sh[col0 + cc]), 0.0f);
-        atomicMax(reinterpret_cast<unsigned int *>(p.out_f32 + (size_t)group * p.ld_f32 + col), __float_as_uint(mx) & 0x7fffffffu);
-    }
-}
-
 // SLOTS tiles in flight per CTA, WG warpgroups (128 threads) working on each: the warpgroups of a slot split the
 // 16-byte chunks of the gather and the 32-column chunks of every epilogue between them.  C: shape policy (above).
 template <class C, int SLOTS, int WG>
@@ -314,7 +206,7 @@ sa_fused_kernel(const SfParams p)
     __shared__ float xs_all[SLOTS * WG][4 * 32];
 
     constexpr int NT = SF_THREADS * SLOTS * WG, ST = SF_THREADS * WG;     // threads per CTA / per slot
-    constexpr int U = WG == 1 ? 4 : (WG == 2 ? 3 : 2);   // gather chunks in flight per thread
+    constexpr int U = WG == 1 ? 4 : 3;                   // gather chunks in flight per thread
     const int tid = threadIdx.x, lane = tid & 31, q = (tid >> 5) & 3;
     const int slot = tid / ST, wg = (tid >> 7) % WG;
     const int r = tid & 127;                             // row of the slot's tile this thread works on
@@ -331,23 +223,20 @@ sa_fused_kernel(const SfParams p)
         mbar_init(smem_u32(&w_bar), 1);
 #pragma unroll
         for (int i = 0; i < SLOTS; i++) mbar_init(smem_u32(&mma_bar[i]), 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        fence_mbar_init_cluster();
         mbar_arrive_expect_tx(smem_u32(&w_bar), cfg.w_total());
         bulk_g2s(smem_u32(wsm), p.w_blob, cfg.w_total(), smem_u32(&w_bar));
     }
-    if (tid < 32) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_smem)), "r"(p.tmem_alloc) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
+    if (tid < 32) tmem_alloc(&tmem_base_smem, p.tmem_alloc);
     for (uint32_t i = tid; i < cfg.ss_total(); i += NT) ss[i] = __ldg(p.ss_blob + i);
     if (cfg.hoist())
         for (int i = tid; i < 3 * kp0; i += NT) {
             const int a3 = i / kp0, k = i - a3 * kp0;
             wxs[i] = k < cfg.c() ? __ldg(p.wx + a3 * cfg.c() + k) : 0.0f;
         }
-    sf_fence_before();
+    tc_fence_before();
     __syncthreads();
-    sf_fence_after();
+    tc_fence_after();
     const uint32_t tmem = tmem_base_smem + (uint32_t)slot * cfg.tmem_cols();
     const uint32_t bar = smem_u32(&mma_bar[slot]);
     mbar_wait_cta(smem_u32(&w_bar), 0);                  // weights landed (async proxy writes, read by UMMA only)
@@ -433,22 +322,12 @@ sa_fused_kernel(const SfParams p)
 #pragma unroll
                 for (int u = 0; u < U; u++) {
                     if (cg0 + u >= nchunk) break;
-                    if (cfg.hoist()) {                                 // relu(z + d . Wx'); padded columns and rows stay 0
-                        const float *w = wxs + (cg0 + u) * 8;
-#pragma unroll
-                        for (int e4 = 0; e4 < 8; e4 += 4) {
-                            const float4 w0 = *reinterpret_cast<const float4 *>(w + e4);
-                            const float4 w1 = *reinterpret_cast<const float4 *>(w + kp0 + e4);
-                            const float4 w2 = *reinterpret_cast<const float4 *>(w + 2 * kp0 + e4);
-                            f[u][e4 + 0] = fmaxf(fmaf(dz, w2.x, fmaf(dy, w1.x, fmaf(dx, w0.x, f[u][e4 + 0]))), 0.0f);
-                            f[u][e4 + 1] = fmaxf(fmaf(dz, w2.y, fmaf(dy, w1.y, fmaf(dx, w0.y, f[u][e4 + 1]))), 0.0f);
-                            f[u][e4 + 2] = fmaxf(fmaf(dz, w2.z, fmaf(dy, w1.z, fmaf(dx, w0.z, f[u][e4 + 2]))), 0.0f);
-                            f[u][e4 + 3] = fmaxf(fmaf(dz, w2.w, fmaf(dy, w1.w, fmaf(dx, w0.w, f[u][e4 + 3]))), 0.0f);
-                        }
-                    }
+                    if (cfg.hoist()) hoist_relu8(f[u], dx, dy, dz, wxs + (cg0 + u) * 8, kp0);   // padded columns and rows stay 0
+                    // spelled out rather than split8_store(): with the chunk offset computed first, the single-slot
+                    // run-time-shape kernel spills 20 more bytes
                     uint32_t hw[4], lw[4], lo_off;
 #pragma unroll
-                    for (int t = 0; t < 4; t++) sf_split_pair(f[u][2 * t], f[u][2 * t + 1], hw[t], lw[t]);
+                    for (int t = 0; t < 4; t++) split_pair(f[u][2 * t], f[u][2 * t + 1], hw[t], lw[t]);
                     const uint32_t off = map0.chunk(cg0 + u, &lo_off);
                     *reinterpret_cast<uint4 *>(buf + off) = make_uint4(hw[0], hw[1], hw[2], hw[3]);
                     *reinterpret_cast<uint4 *>(buf + off + lo_off) = make_uint4(lw[0], lw[1], lw[2], lw[3]);
@@ -459,15 +338,15 @@ sa_fused_kernel(const SfParams p)
 #pragma unroll (C::kStatic ? SF_MAX_LAYERS : 1)
         for (int l = 0; l < cfg.nl(); l++) {
             // operand written with ordinary stores -> make it visible to the tensor-core (async) proxy
-            sf_fence_async_smem();
-            sf_fence_before();
-            sf_bar_sync(slot_bar, ST);
+            fence_async_smem();
+            tc_fence_before();
+            bar_sync(slot_bar, ST);
             SF_T(1 + 4 * l);                                           // barrier
             if (issuer_warp) {
-                sf_fence_after();
+                tc_fence_after();
                 // one MMA per k-step covers the whole layer width: a tcgen05.mma costs ~N/2 cycles plus a fixed
                 // per-instruction part, so narrower MMAs only add overhead (measured in round 1)
-                const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(cfg.npad(l) >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
+                const uint32_t idesc = umma_idesc_bf16(cfg.npad(l));
                 const uint32_t tmem_u = tmem_base_smem + (uint32_t)slot_u * cfg.tmem_cols();
                 const uint32_t abase = smem_u32(smem) + (uint32_t)slot_u * cfg.abuf_bytes();
                 const uint32_t wbase = smem_u32(wsm) + cfg.w_off(l);
@@ -476,46 +355,38 @@ sa_fused_kernel(const SfParams p)
                 // descriptors advance by (bytes >> 4) in their address field; shared memory < 256 KiB: no carry out of it
 #pragma unroll (C::kStatic ? 4 : 1)
                 for (int kb = 0; kb < nfull; kb++) {
-                    const uint64_t a_hi = sf_desc(abase + (uint32_t)kb * (2u * 128u * 128u), 128);
-                    const uint64_t b_hi = sf_desc(wbase + (uint32_t)kb * ((uint32_t)cfg.npad(l) * 128u), 128);
+                    const uint64_t a_hi = umma_desc(abase + (uint32_t)kb * (2u * 128u * 128u), 128);
+                    const uint64_t b_hi = umma_desc(wbase + (uint32_t)kb * ((uint32_t)cfg.npad(l) * 128u), 128);
                     const uint64_t a_lo = a_hi + ((128u * 128u) >> 4), b_lo = b_hi + (cfg.w_half(l) >> 4);
 #pragma unroll
                     for (int kin = 0; kin < 4; kin++) {
-                        if (elect_one()) {
-                            sf_mma(tmem_u, a_hi + 2 * kin, b_hi + 2 * kin, idesc, acc);
-                            sf_mma(tmem_u, a_lo + 2 * kin, b_hi + 2 * kin, idesc, 1u);
-                            sf_mma(tmem_u, a_hi + 2 * kin, b_lo + 2 * kin, idesc, 1u);
-                        }
+                        if (elect_one()) umma_bf16x3(tmem_u, a_hi + 2 * kin, a_lo + 2 * kin, b_hi + 2 * kin, b_lo + 2 * kin, idesc, acc);
                         acc = 1u;
                     }
                 }
                 if (rbt) {
-                    const uint64_t a_hi = sf_desc(abase + (uint32_t)nfull * (2u * 128u * 128u), rbt);
-                    const uint64_t b_hi = sf_desc(wbase + (uint32_t)nfull * ((uint32_t)cfg.npad(l) * 128u), rbt);
+                    const uint64_t a_hi = umma_desc(abase + (uint32_t)nfull * (2u * 128u * 128u), rbt);
+                    const uint64_t b_hi = umma_desc(wbase + (uint32_t)nfull * ((uint32_t)cfg.npad(l) * 128u), rbt);
                     const uint64_t a_lo = a_hi + ((128u * (uint32_t)rbt) >> 4), b_lo = b_hi + (cfg.w_half(l) >> 4);
                     const int nt = rbt == 128 ? 3 : (rbt >> 5);              // 16-wide k-steps of the tail block
 #pragma unroll (C::kStatic ? 3 : 1)
                     for (int kin = 0; kin < nt; kin++) {
-                        if (elect_one()) {
-                            sf_mma(tmem_u, a_hi + 2 * kin, b_hi + 2 * kin, idesc, acc);
-                            sf_mma(tmem_u, a_lo + 2 * kin, b_hi + 2 * kin, idesc, 1u);
-                            sf_mma(tmem_u, a_hi + 2 * kin, b_lo + 2 * kin, idesc, 1u);
-                        }
+                        if (elect_one()) umma_bf16x3(tmem_u, a_hi + 2 * kin, a_lo + 2 * kin, b_hi + 2 * kin, b_lo + 2 * kin, idesc, acc);
                         acc = 1u;
                     }
                 }
-                if (elect_one()) sf_commit(smem_u32(&mma_bar[slot_u]));
+                if (elect_one()) umma_commit(smem_u32(&mma_bar[slot_u]));
                 __syncwarp();
                 SF_T(2 + 4 * l);                                       // MMA issue
                 // ONE warp of the slot polls the mbarrier; the others sleep at the slot's named barrier (a hardware
                 // barrier costs no issue slots -- the all-warps poll loop was a quarter of the kernel's instructions)
                 mbar_wait_cta(bar, mma_phase);                       // MMAs done: accumulator ready, operand buffer free
-                sf_fence_before();
+                tc_fence_before();
             }
-            sf_bar_sync(slot_bar, ST);
+            bar_sync(slot_bar, ST);
             mma_phase ^= 1u;
             SF_T(3 + 4 * l);                                           // MMA wait
-            sf_fence_after();
+            tc_fence_after();
             // ---- epilogue of layer l
             const float *sc = ss + cfg.ss_off(l);
             const float *sh = sc + cfg.sspad(l);
@@ -527,7 +398,7 @@ sa_fused_kernel(const SfParams p)
             for (int ci = wg; ci < nchunks; ci += WG) {
                 const int c0 = ci * 32;
                 uint32_t rr[32];
-                sf_tmem_ld32(tmem + ((uint32_t)(q * 32) << 16) + (uint32_t)c0, rr);
+                tmem_ld32(tmem + ((uint32_t)(q * 32) << 16) + (uint32_t)c0, rr);
                 float v[32];
                 if (pool_first) {
 #pragma unroll
@@ -547,44 +418,29 @@ sa_fused_kernel(const SfParams p)
 #pragma unroll
                     for (int j8 = 0; j8 < 32; j8 += 8) {
                         if (c0 + j8 >= cfg.kp(l + 1)) break;
-                        uint32_t hw[4], lw[4], lo_off;
-#pragma unroll
-                        for (int t = 0; t < 4; t++) sf_split_pair(v[j8 + 2 * t], v[j8 + 2 * t + 1], hw[t], lw[t]);
+                        uint32_t lo_off;
                         const uint32_t off = mapn.chunk((c0 + j8) >> 3, &lo_off);
-                        *reinterpret_cast<uint4 *>(buf + off) = make_uint4(hw[0], hw[1], hw[2], hw[3]);
-                        *reinterpret_cast<uint4 *>(buf + off + lo_off) = make_uint4(lw[0], lw[1], lw[2], lw[3]);
+                        split8_store(v + j8, buf + off, buf + off + lo_off);
                     }
                 } else if (compact) {
-                    if (pool_first) sf_pool_atomic8<true>(p, v, lane, c0, cfg.nout(l), sc, sh, my_group, my_ok);
-                    else sf_pool_atomic8<false>(p, v, lane, c0, cfg.nout(l), sc, sh, my_group, my_ok);
+                    if (pool_first) pool_units<true>(p, v, lane, c0, cfg.nout(l), sc, sh, my_group, my_ok);
+                    else pool_units<false>(p, v, lane, c0, cfg.nout(l), sc, sh, my_group, my_ok);
                 } else if (pool_first) {
-                    switch (cfg.ns()) {
-                        case 8: sf_pool_store<8, true>(p, v, lane, q, tile, c0, cfg.nout(l), xs, wg_bar, sc, sh); break;
-                        case 16: sf_pool_store<16, true>(p, v, lane, q, tile, c0, cfg.nout(l), xs, wg_bar, sc, sh); break;
-                        case 32: sf_pool_store<32, true>(p, v, lane, q, tile, c0, cfg.nout(l), xs, wg_bar, sc, sh); break;
-                        case 64: sf_pool_store<64, true>(p, v, lane, q, tile, c0, cfg.nout(l), xs, wg_bar, sc, sh); break;
-                        default: sf_pool_store<128, true>(p, v, lane, q, tile, c0, cfg.nout(l), xs, wg_bar, sc, sh); break;
-                    }
+                    pool_rows<true>(cfg.ns(), p, p.cnt, v, lane, q, tile, c0, cfg.nout(l), sc, sh, xs, wg_bar);
                 } else {
-                    switch (cfg.ns()) {
-                        case 8: sf_pool_store<8, false>(p, v, lane, q, tile, c0, cfg.nout(l), xs, wg_bar, sc, sh); break;
-                        case 16: sf_pool_store<16, false>(p, v, lane, q, tile, c0, cfg.nout(l), xs, wg_bar, sc, sh); break;
-                        case 32: sf_pool_store<32, false>(p, v, lane, q, tile, c0, cfg.nout(l), xs, wg_bar, sc, sh); break;
-                        case 64: sf_pool_store<64, false>(p, v, lane, q, tile, c0, cfg.nout(l), xs, wg_bar, sc, sh); break;
-                        default: sf_pool_store<128, false>(p, v, lane, q, tile, c0, cfg.nout(l), xs, wg_bar, sc, sh); break;
-                    }
+                    pool_rows<false>(cfg.ns(), p, p.cnt, v, lane, q, tile, c0, cfg.nout(l), sc, sh, xs, wg_bar);
                 }
             }
-            sf_fence_before();                                         // TMEM reads done before the next MMAs overwrite it
+            tc_fence_before();                                         // TMEM reads done before the next MMAs overwrite it
             SF_T(4 + 4 * l);                                           // epilogue
         }
     }
 
-    sf_fence_before();
+    tc_fence_before();
     __syncthreads();
     if (tid < 32) {
-        sf_fence_after();
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base_smem), "r"(p.tmem_alloc) : "memory");
+        tc_fence_after();
+        tmem_dealloc(tmem_base_smem, p.tmem_alloc);
     }
 }
 
@@ -592,25 +448,9 @@ sa_fused_kernel(const SfParams p)
 
 using namespace ssd3d;
 
-// Operand layout of a layer with padded K = kp: nfull 64-wide k-blocks of 128-byte rows + a tail block whose rows
-// are 32 / 64 / 128 bytes for a remainder of 16 / 32 / 48 columns (must match params._k_blocks).
-static void sf_k_blocks(int kp, int *nfull, int *rbt)
-{
-    *nfull = kp / 64;
-    const int rem = kp % 64;
-    *rbt = rem == 0 ? 0 : (rem <= 16 ? 32 : (rem <= 32 ? 64 : 128));
-}
-static size_t sf_abuf_bytes(int kp)                       // { hi | lo } tiles of 128 rows per block, 1 KiB granular
-{
-    int nfull, rbt;
-    sf_k_blocks(kp, &nfull, &rbt);
-    return ((size_t)nfull * 2 * 128 * 128 + (size_t)2 * 128 * rbt + 1023) / 1024 * 1024;
-}
 static size_t sf_wimg_bytes(int kp, int npad)              // one half (hi or lo) of a layer's weight image
 {
-    int nfull, rbt;
-    sf_k_blocks(kp, &nfull, &rbt);
-    return (size_t)npad * (nfull * 128 + rbt);
+    return (size_t)npad * ((kp / 64) * 128 + sf_rbt_of(kp));
 }
 
 struct SfPlan { size_t abuf, w, ssf; int maxn; };
@@ -623,7 +463,7 @@ static bool sf_plan(int k_in, int nl, const int *nout, SfPlan *pl)      // k_in:
     for (int l = 0; l < nl; l++) {
         const int npad = (nout[l] + 15) / 16 * 16;
         if (npad > 256) return false;
-        const size_t a = sf_abuf_bytes(kp);
+        const size_t a = sf_abuf_of(kp);
         if (a > pl->abuf) pl->abuf = a;
         pl->w += 2 * sf_wimg_bytes(kp, npad);
         pl->ssf += (size_t)2 * ((npad + 31) / 32 * 32);
@@ -636,23 +476,25 @@ static size_t sf_total(const SfPlan &pl, int slots) { return slots * pl.abuf + p
 constexpr size_t SF_SMEM_MAX = 226 * 1024;
 constexpr size_t SF_SMALL = 36 * 1024;                     // <= this: single-slot CTAs, up to 6 per SM
 
-// Developer build only (-DSSD3D_DEV_HOOKS, csrc/ssd3d_dev.h): override the slot / warpgroup shape from a probe script.
-// The shipped library has no such state.
+// Developer build only (-DSSD3D_DEV_HOOKS, `python 3dssd_b200/build.py dev`, called by tools/fused_probe.py dyn=1):
+// launch the run-time-shape kernel even where a compile-time-shape twin exists, for A/B timing of the two.  The shipped
+// library has no such state.
 #ifdef SSD3D_DEV_HOOKS
-static int g_sf_slots = 0, g_sf_wg = 0, g_sf_dynamic = 0;
-extern "C" void ssd3d_dev_set_fused(int slots, int wg) { g_sf_slots = slots; g_sf_wg = wg; }
-extern "C" void ssd3d_dev_set_fused_dynamic(int on) { g_sf_dynamic = on; }   // force the run-time-shape kernel (A/B timing)
+static int g_sf_dynamic = 0;
+extern "C" void ssd3d_dev_set_fused_dynamic(int on) { g_sf_dynamic = on; }
 #else
-constexpr int g_sf_slots = 0, g_sf_wg = 0, g_sf_dynamic = 0;
+constexpr int g_sf_dynamic = 0;
 #endif
 
-// Slots per CTA for a stack: 1 for small stacks (several CTAs per SM), else as many as fit one SM (<= 3).
+// Slots per CTA for a stack: 1 for small stacks (several CTAs per SM), else as many as fit one SM (<= 3).  A slot of a
+// multi-slot CTA has two warpgroups: on the layer-2 stacks 3 x 2 beat the slot x warpgroup shapes 4 x 1, 3 x 1, 2 x 2
+// and 2 x 4.
 static int sf_slots(const SfPlan &pl)
 {
     if (sf_total(pl, 1) <= SF_SMALL) return 1;
     int cols = 32;
     while (cols < pl.maxn) cols *= 2;
-    int s = g_sf_slots > 0 ? (g_sf_slots > 4 ? 4 : g_sf_slots) : 3;
+    int s = 3;
     while (s > 1 && (sf_total(pl, s) > SF_SMEM_MAX || s * cols > 512)) s--;
     return s;
 }
@@ -680,16 +522,16 @@ static cudaError_t sf_launch(const SfParams &p, size_t smem, int per_sm, cudaStr
 
 // The hoisted two-conv stacks of the shipped 3DSSD configuration (configs/kitti/3dssd/3dssd.yaml:47-52) have compile-time
 // twins of the kernel: layer 1 [16 -> 16 -> 32] x32 and [32 -> 32 -> 64] x64 neighbours, layer 2 [64 -> 64 -> 128] x32 and
-// [64 -> 96 -> 128] x64.  Returns false when (shape, slots, warpgroups) has no twin: the caller takes the dynamic kernel.
-static bool sf_launch_static(const SfParams &p, int slots, int wg, size_t smem, int per_sm, cudaStream_t st, cudaError_t *e)
+// [64 -> 96 -> 128] x64.  Returns false when (shape, slots) has no twin: the caller takes the dynamic kernel.
+static bool sf_launch_static(const SfParams &p, int slots, size_t smem, int per_sm, cudaStream_t st, cudaError_t *e)
 {
     if (!p.hoist || p.nl != 2) return false;
     const int k0 = p.c, n0 = p.nout[0], n1 = p.nout[1], ns = p.ns;
-    if (slots == 1 && wg == 1) {
+    if (slots == 1) {
         if (k0 == 16 && n0 == 16 && n1 == 32 && ns == 32) { *e = sf_launch<SfStat<16, 16, 32, 32>, 1, 1>(p, smem, per_sm, st); return true; }
         if (k0 == 32 && n0 == 32 && n1 == 64 && ns == 64) { *e = sf_launch<SfStat<32, 32, 64, 64>, 1, 1>(p, smem, per_sm, st); return true; }
     }
-    if (slots == 3 && wg == 2) {
+    if (slots == 3) {
         if (k0 == 64 && n0 == 64 && n1 == 128 && ns == 32) { *e = sf_launch<SfStat<64, 64, 128, 32>, 3, 2>(p, smem, per_sm, st); return true; }
         if (k0 == 64 && n0 == 96 && n1 == 128 && ns == 64) { *e = sf_launch<SfStat<64, 96, 128, 64>, 3, 2>(p, smem, per_sm, st); return true; }
     }
@@ -737,7 +579,8 @@ static int sa_mlp_fused_impl(int b, int n, int c, int m, int nsample, const floa
         p.kp[l] = kprev;
         p.nout[l] = nout[l];
         p.npad[l] = (nout[l] + 15) / 16 * 16;
-        sf_k_blocks(p.kp[l], &p.nfull[l], &p.rbt[l]);
+        p.nfull[l] = p.kp[l] / 64;
+        p.rbt[l] = sf_rbt_of(p.kp[l]);
         p.w_off[l] = woff;
         p.w_half[l] = (uint32_t)sf_wimg_bytes(p.kp[l], p.npad[l]);
         woff += 2 * p.w_half[l];
@@ -766,15 +609,12 @@ static int sa_mlp_fused_impl(int b, int n, int c, int m, int nsample, const floa
         if (per_sm < 1) per_sm = 1;
         if (per_sm > 6) per_sm = 6;                                   // 6 x 128 threads x 80 registers
     }
-    const int wg = slots == 1 ? 1 : (g_sf_wg > 0 ? g_sf_wg : 2);
     cudaStream_t st = (cudaStream_t)stream;
     cudaError_t e = cudaSuccess;
-    if (g_sf_dynamic || !sf_launch_static(p, slots, wg, smem, per_sm, st, &e))
+    if (g_sf_dynamic || !sf_launch_static(p, slots, smem, per_sm, st, &e))
         e = slots == 1 ? sf_launch<SfDyn, 1, 1>(p, smem, per_sm, st)
-          : slots == 2 ? (wg == 4 ? sf_launch<SfDyn, 2, 4>(p, smem, per_sm, st) : wg == 1 ? sf_launch<SfDyn, 2, 1>(p, smem, per_sm, st)
-                                                                                           : sf_launch<SfDyn, 2, 2>(p, smem, per_sm, st))
-          : slots == 3 ? (wg == 1 ? sf_launch<SfDyn, 3, 1>(p, smem, per_sm, st) : sf_launch<SfDyn, 3, 2>(p, smem, per_sm, st))
-                       : sf_launch<SfDyn, 4, 1>(p, smem, per_sm, st);
+          : slots == 2 ? sf_launch<SfDyn, 2, 2>(p, smem, per_sm, st)
+                       : sf_launch<SfDyn, 3, 2>(p, smem, per_sm, st);
     if (e != cudaSuccess) return cuda_status(e, "sa_mlp_fused attr");
 #ifdef SF_PROFILE
     {

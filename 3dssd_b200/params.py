@@ -132,7 +132,7 @@ def fold(params, scope, bn, device):
 def _k_blocks(kp):
     """Operand layout of the fused kernel for a padded K: (nfull, rbt) = number of 64-wide k-blocks (128-byte rows) and
     the row bytes of the tail block -- 0 / 32 / 64 / 128 for a remainder of 0 / 16 / 32 / 48 columns (must match
-    sf_k_blocks in csrc/sa_fused.cu)."""
+    sf_rbt_of in csrc/sa_fused.cu)."""
     rem = kp % 64
     return kp // 64, 0 if rem == 0 else (32 if rem <= 16 else (64 if rem <= 32 else 128))
 

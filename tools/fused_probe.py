@@ -1,8 +1,8 @@
 """Runs the fused SA-scale kernel on layer-1 / layer-2 shaped inputs (for timing and ncu captures).
-usage: python tools/fused_probe.py [case-index ...] [hoist=1] [dyn=1] [slots=S wg=W]
+usage: python tools/fused_probe.py [case-index ...] [hoist=1] [dyn=1]
   hoist=1 (default)  the hoisted form the model runs (first conv in the per-point table); hoist=0 the literal 3-conv stack
-  dyn=1 / slots / wg developer build only (SSD3D_LIB=3dssd_b200/libssd3d_dev.so): force the run-time-shape kernel /
-                     the slot x warpgroup shape, for A/B timing against the compile-time-shape kernels"""
+  dyn=1              developer build only (SSD3D_LIB=3dssd_b200/libssd3d_dev.so): force the run-time-shape kernel, for
+                     A/B timing against the compile-time-shape kernels"""
 import importlib
 import os
 import sys
@@ -28,11 +28,10 @@ def main():
     dev = torch.device("cuda:0")
     sel = [int(a) for a in sys.argv[1:] if "=" not in a] or range(len(CASES))
     kv = dict(a.split("=") for a in sys.argv[1:] if "=" in a)
-    if "slots" in kv or "wg" in kv or "dyn" in kv:   # developer build only (nvcc -DSSD3D_DEV_HOOKS, loaded through SSD3D_LIB)
+    if "dyn" in kv:   # developer build only (nvcc -DSSD3D_DEV_HOOKS, loaded through SSD3D_LIB)
         import ctypes
         dl = ctypes.CDLL(pkg.LIB_PATH)
-        dl.ssd3d_dev_set_fused(int(kv.get("slots", 0)), int(kv.get("wg", 0)))
-        dl.ssd3d_dev_set_fused_dynamic(int(kv.get("dyn", 0)))
+        dl.ssd3d_dev_set_fused_dynamic(int(kv["dyn"]))
     hoist = int(kv.get("hoist", 1))
     rng = np.random.default_rng(0)
     B = 8

@@ -11,9 +11,8 @@ timeout 300 python tools/time_ops.py $O/r02_time_ops.json > $O/time_ops.log 2>&1
 # phase profiles of the tensor-core kernels (instrumented build)
 SSD3D_LIB=3dssd_b200/libssd3d_prof.so timeout 300 python tools/tc_probe.py 9 10 11 1 2 3 > $O/tc_prof.log 2>&1
 SSD3D_LIB=3dssd_b200/libssd3d_prof.so timeout 300 python tools/fused_probe.py 0 1 2 3 > $O/fused_prof.log 2>&1
-# A/B: compile-time-shape kernels vs the run-time-shape kernel, and slot shapes for the layer-2 stacks (dev-hook build)
+# A/B: compile-time-shape kernels vs the run-time-shape kernel (dev-hook build)
 for a in "" "dyn=1" ; do SSD3D_LIB=3dssd_b200/libssd3d_dev.so timeout 120 python tools/fused_probe.py 0 1 2 3 $a >> $O/fused_ab.log 2>&1; done
-for a in "dyn=1 slots=4 wg=1" "dyn=1 slots=3 wg=1" "dyn=1 slots=2 wg=2" "dyn=1 slots=2 wg=4"; do SSD3D_LIB=3dssd_b200/libssd3d_dev.so timeout 120 python tools/fused_probe.py 2 3 $a >> $O/fused_ab.log 2>&1; done
 # sanitizer (small shapes)
 timeout 900 compute-sanitizer --tool memcheck --error-exitcode 9 python tools/sanitize_probe.py > $O/r02_sanitizer_memcheck.txt 2>&1; echo "exit $?" >> $O/r02_sanitizer_memcheck.txt
 timeout 900 compute-sanitizer --tool racecheck --error-exitcode 9 python tools/sanitize_probe.py > $O/r02_sanitizer_racecheck.txt 2>&1; echo "exit $?" >> $O/r02_sanitizer_racecheck.txt
